@@ -46,7 +46,27 @@ def parse():
     ap.add_argument("--locality", type=float, default=0.9)
     ap.add_argument("--window", type=int, default=8192)
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / e2e / reference_gpu / other-config legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's forward and backward aggregation as DIR/fwd_aggregate.npy "
+                         "and DIR/bwd_aggregate.npy (float32; a fixed seeded sample of rows when the arrays exceed 60 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return args
+
+
+DUMP_BYTES = 60_000_000     # all arrays --dump-outputs writes, together
+
+
+def dump_rows(num_rows, row_bytes, n_arrays):
+    """Row ids --dump-outputs writes: every row when the arrays fit in DUMP_BYTES, else a fixed seeded sample (sorted),
+    the same for every run and build with the same graph size."""
+    cap = DUMP_BYTES // (row_bytes * n_arrays)
+    if num_rows <= cap:
+        return torch.arange(num_rows)
+    return torch.randperm(num_rows, generator=torch.Generator().manual_seed(0))[:cap].sort().values
 
 
 def peaks():
@@ -373,6 +393,25 @@ def main():
     barrier()
     launches = kernels.launch_count - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # out_f / out_b still hold the last timed step's results: the legs below reuse these buffers
+        import numpy as np
+
+        rows = dump_rows(n, FEAT * out_f.element_size(), 2)
+        dumped = {}
+        for name, out in (("fwd_aggregate", out_f), ("bwd_aggregate", out_b)):
+            if world > 1:   # every rank holds a contiguous, ascending range of rows
+                mine = rows[(rows >= lo) & (rows < hi)]
+                parts = [None] * world
+                dist.all_gather_object(parts, out[(mine - lo).to(dev)].cpu())
+                dumped[name] = torch.cat(parts)
+            else:
+                dumped[name] = out[rows.to(dev)].cpu()
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.numpy())
+        del dumped
     ms_total = t_beg.elapsed_time(t_end)
     ms_fwd_kernel = sum(a.elapsed_time(b) for a, b in kev) / args.steps
     ms_fwd_own = ms_fwd_kernel

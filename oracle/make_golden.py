@@ -147,6 +147,109 @@ def make_updates_golden():
     print("wrote", os.path.join(GOLD, "ref_updates.npz"), len(out), "arrays")
 
 
+def live_graph(n, e, seed):
+    """Random directed graph of ``min(e, n*n)`` distinct edges (self loops allowed) for the randomized oracle tests."""
+    rng = np.random.default_rng(seed)
+    key = rng.choice(n * n, size=min(e, n * n), replace=False)
+    return (key // n).astype(np.int32), (key % n).astype(np.int32)
+
+
+def live_gcn_inputs(feat, n, e, seed):
+    """Inputs of ``test_aggregation_oracle_equals_reference_kernels_live``: a random graph plus a star around vertex 0
+    (one long row and many short ones), no self loops; ``(src, dst, edge_weight_by_eid, norm [N,1], h, grad_in)``."""
+    src, dst = live_graph(n, e, seed)
+    star = np.arange(1, n, dtype=np.int32)
+    k = np.unique(np.concatenate([src.astype(np.int64) * n + dst, star.astype(np.int64) * n, star.astype(np.int64)]))
+    src, dst = (k // n).astype(np.int32), (k % n).astype(np.int32)
+    keep = src != dst
+    src, dst = src[keep], dst[keep]
+    rng = np.random.default_rng(seed + 7)
+    w = rng.uniform(0.1, 1.0, size=src.shape[0]).astype(np.float32)
+    norm = rng.uniform(0.2, 1.0, size=(n, 1)).astype(np.float32)
+    h = rng.standard_normal((n, feat)).astype(np.float32)
+    gin = rng.standard_normal((n, feat)).astype(np.float32)
+    return src, dst, w, norm, h, gin
+
+
+def live_gat_inputs(heads, dim, n, e, seed):
+    """Inputs of ``test_stock_gat_oracle_equals_reference_kernels_live``: ``(src, dst, el, er, feat, grad_out)``."""
+    src, dst = live_graph(n, e, seed)
+    keep = src != dst
+    src, dst = src[keep], dst[keep]
+    rng = np.random.default_rng(seed + 11)
+    f32 = lambda *s: rng.standard_normal(s).astype(np.float32)
+    return (src, dst) + (f32(n, heads, 1), f32(n, heads, 1), f32(n, heads, dim), f32(n, heads, dim))
+
+
+LIVE_GCN_CASES = (("gcn_f16", 16, False), ("gcn_f100", 100, False), ("gcn_f128", 128, False), ("gcnw_f7", 7, True))
+LIVE_GCN_GRAPHS = ((12, 30, 0), (100, 1500, 1), (400, 6000, 2))
+LIVE_GAT_CASES = (("gat_h2d4", 2, 4), ("gat_h8d16", 8, 16))
+LIVE_GAT_GRAPHS = ((30, 150, 0), (200, 2500, 1))
+
+
+def sample_rows(num_rows, row_width, seed, budget=2048):
+    """Rows of one output kept in the fixture: the first and the last row plus a seeded sample, ~``budget`` values."""
+    k = min(num_rows, max(4, budget // max(row_width, 1)))
+    pick = np.random.default_rng(seed).choice(num_rows, size=k, replace=False)
+    return np.unique(np.concatenate([[0, num_rows - 1], pick])).astype(np.int32)
+
+
+def make_live_golden():
+    """The reference kernels' outputs on the seeded inputs of the randomized oracle tests (``ref_kernels_live.npz``).
+
+    The emitted kernels read only ``row_offsets``, ``column_indices`` and ``eids`` of a CSR (``node_ids`` is never
+    indexed), and ``oracle/structure.py`` reproduces those three arrays of the reference's ``CSR::CSR`` bit for bit
+    (``ref_structure.npz``), so the kernels run on the oracle's CSRs here.  Only a seeded sample of rows of every output
+    is stored (``<key>/rows`` holds the row ids) to keep the fixture small; the inputs are rebuilt from their seeds."""
+    from oracle import structure as S
+
+    out = {}
+
+    def run(case, tensors, grads, src, dst, n):
+        kernels, lib = RE.load_case(case)
+        ne = src.shape[0]
+        fwd, bwd = S.forward_csr(src, dst, n), S.backward_csr(src, dst, n)
+        for kern in kernels:
+            for name, vt, shp in zip(kern["args"], kern["arg_types"], kern["arg_shapes"]):
+                if name not in tensors:
+                    lead = ne if vt == "EDGE" else n
+                    tensors[name] = np.zeros([lead] + shp, np.float32) if name in kern["rets"] else grads.pop(0)
+            RE.run_reference_kernel(lib, kern, tensors, fwd if kern["parallel_mode"] == "DstParallel" else bwd, n)
+        return kernels
+
+    def store(key, arr, seed):
+        arr = arr.reshape(arr.shape[0], -1)
+        rows = sample_rows(arr.shape[0], arr.shape[1], seed)
+        out[f"{key}/rows"] = rows
+        out[key] = arr[rows]
+
+    for case, feat, weighted in LIVE_GCN_CASES:
+        for n, e, seed in LIVE_GCN_GRAPHS:
+            src, dst, w, norm, h, gin = live_gcn_inputs(feat, n, e, seed)
+            tensors = {"Vhinb": h, "Vnormcen": norm, "Vnorminb": norm}
+            if weighted:
+                tensors["Vedge_weight"] = w.reshape(-1, 1).copy()
+            kernels = run(case, tensors, [gin], src, dst, n)
+            for kern in kernels:
+                store(f"gcn/{case}/{n}_{e}_{seed}/{kern['direction']}", tensors[kern["rets"][0]], seed)
+    for case, heads, dim in LIVE_GAT_CASES:
+        for n, e, seed in LIVE_GAT_GRAPHS:
+            src, dst, el, er, feat, gout = live_gat_inputs(heads, dim, n, e, seed)
+            tensors = {"Velinb": el, "Vercen": er, "Vfeat_srcinb": feat}
+            k0, k1, k2 = run(case, tensors, [gout], src, dst, n)
+            rets = [tensors[r] for r in k2["rets"]]
+            d_feat = [r for r in rets if r.shape[-1] == dim and r.ndim == 3 and r.shape[1] == heads][0]
+            small = [r for r in rets if r.shape[-1] == 1]
+            key = f"gat/{case}/{n}_{e}_{seed}"
+            out[f"{key}/d_feat_abs_mean"] = np.float64(np.abs(d_feat.astype(np.float64)).mean())
+            for role, arr in (("v3", tensors[k0["rets"][0]]), ("v4", tensors[k0["rets"][1]]), ("out", tensors[k1["rets"][0]]),
+                              ("d_feat", d_feat), ("d_el", max(small, key=lambda x: float(np.abs(x).max()))),
+                              ("d_er", min(small, key=lambda x: float(np.abs(x).max())))):
+                store(f"{key}/{role}", arr, seed)
+    np.savez_compressed(os.path.join(GOLD, "ref_kernels_live.npz"), **out)
+    print("wrote", os.path.join(GOLD, "ref_kernels_live.npz"), len(out), "arrays")
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     make_updates_golden()
@@ -204,6 +307,7 @@ def main():
         el, er, feat = f32(n, hh, 1), f32(n, hh, 1), f32(n, hh, dd)
         run_case(case, {"Velinb": el, "Vercen": er, "Vfeat_srcinb": feat}, [f32(n, hh, dd)])
     make_pcsr_golden()
+    make_live_golden()
     np.savez_compressed(os.path.join(GOLD, "ref_kernels.npz"), **kout)
     print("wrote", os.path.join(GOLD, "ref_structure.npz"), "and ref_kernels.npz:", len(kout), "arrays")
 

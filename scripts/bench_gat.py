@@ -1,7 +1,7 @@
 """Device time of the fused edge-softmax kernels on the arxiv-shaped graph (config 3): raw C-ABI calls on
 preallocated buffers, 20 back-to-back iterations between two CUDA events (no per-call Python allocation)."""
 import ctypes, json, os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import _lib, ops_gat
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.utils import synthetic

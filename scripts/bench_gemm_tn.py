@@ -1,10 +1,11 @@
 """Device time of kernels.gemm_tn against torch.mm(a.t(), b) on the weight-gradient shapes of the TGCN cell (config 4)."""
 import json
+import os
 import sys
 
 import torch
 
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import kernels  # noqa: E402
 
 dev = torch.device("cuda")

@@ -1,6 +1,6 @@
 """Profiling driver: a few launches of the F=100 forward aggregation on the config-5 graph."""
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import kernels
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.utils import synthetic

@@ -1,6 +1,6 @@
 """Profiling driver: fused edge-softmax GAT forward + backward on the arxiv-shaped graph (config 3)."""
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.ops_gat import gat_edge_softmax_aggregate
 from stgraph_b200.utils import synthetic

@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.nn.pytorch import GATConv
 from stgraph_b200.utils import synthetic

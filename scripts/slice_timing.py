@@ -1,7 +1,7 @@
 """Single-GPU timing of one rank's share of the 8-way partitioned aggregation (no communication):
 own-source pass, halo-source pass, alone and concurrently -- isolates kernel efficiency at slice size."""
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import _lib, kernels
 from stgraph_b200.dist.partition import edge_balanced_bounds
 from stgraph_b200.graph import StaticGraph
@@ -17,7 +17,6 @@ x = torch.randn(n, F, device=dev)
 csr = g._forward_graph
 bounds = edge_balanced_bounds(csr.row_offset, P)
 keep = []
-import os
 USE_QUEUE = os.environ.get('STG_SLICE_QUEUE', '1') != '0'
 
 def mkview(ro, cols, n_rows):

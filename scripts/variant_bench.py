@@ -1,6 +1,6 @@
 """A/B timing of the aggregation kernel variants on the config-5 graph (F=100 and F=128)."""
 import os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import kernels
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.utils import synthetic

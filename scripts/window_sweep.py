@@ -1,6 +1,6 @@
 """Experiment: how does the aggregation time respond to neighbour locality (Laplace window)?"""
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stgraph_b200 import kernels
 from stgraph_b200.graph import StaticGraph
 from stgraph_b200.utils import synthetic

@@ -1,32 +1,34 @@
-"""Live pinning of the structure oracle against the reference's OWN code, on random inputs.
+"""Pinning of the oracle against the reference's OWN code, on random inputs.
 
-``oracle/build_ref.py`` compiles the reference's ``csr.cu`` and ``pcsr.cu`` from where they lie into
-``oracle/_ref/*.so`` (host code; no GPU needed to run it).  Where those libraries exist (the build container, and
-the GPU box, to which ``oracle/_ref`` travels) these tests drive them on seeded random graphs / streams and demand
-bit-identical arrays from ``oracle/structure.py`` -- the committed fixtures in ``tests/golden`` are two such runs.
+Aggregation and GAT: the outputs of the CUDA kernels the reference's code generator emits, run on these tests' seeded
+inputs, are stored in ``tests/golden/ref_kernels_live.npz`` (``oracle/make_golden.py``); the tests rebuild the inputs
+from their seeds and compare the oracle with the stored rows.
+
+Structure: ``oracle/build_ref.py`` compiles the reference's ``csr.cu`` and ``pcsr.cu`` from its sources into
+``oracle/_ref/*.so`` (host code; no GPU needed to run it).  Where those libraries are built, these tests drive them on
+seeded random graphs / streams and demand bit-identical arrays from ``oracle/structure.py``; elsewhere they skip, and
+the committed fixtures ``tests/golden/ref_structure.npz`` / ``ref_pcsr.npz`` (tests/test_golden_oracle.py) are such runs.
 """
 import os
 
 import numpy as np
 import pytest
+import torch
 
+from oracle import aggregate as A
+from oracle import make_golden as MG
 from oracle import ref_emulate as RE
 from oracle import structure as S
 
+GOLD = os.path.join(os.path.dirname(__file__), "golden")
 HAVE_CSR = os.path.exists(os.path.join(RE.REF_DIR, "ref_csr.so"))
 HAVE_PCSR = os.path.exists(os.path.join(RE.REF_DIR, "ref_pcsr.so"))
 
 
-def _graph(n, e, seed):
-    rng = np.random.default_rng(seed)
-    key = rng.choice(n * n, size=min(e, n * n), replace=False)
-    return (key // n).astype(np.int32), (key % n).astype(np.int32)
-
-
-@pytest.mark.skipif(not HAVE_CSR, reason="oracle/_ref/ref_csr.so not built (needs /root/reference)")
+@pytest.mark.skipif(not HAVE_CSR, reason="oracle/_ref/ref_csr.so not built (oracle/build_ref.py needs the reference's sources)")
 @pytest.mark.parametrize("n,e,seed", [(1, 0, 0), (2, 1, 1), (7, 20, 2), (50, 400, 3), (300, 5000, 4), (1000, 3000, 5)])
 def test_static_structure_oracle_equals_reference_csr_builder(n, e, seed):
-    src, dst = _graph(n, e, seed)
+    src, dst = MG.live_graph(n, e, seed)
     if e == 0:
         src, dst = np.zeros(0, np.int32), np.zeros(0, np.int32)
     w = np.random.default_rng(seed + 100).uniform(0.1, 1.0, size=src.shape[0]).astype(np.float32)
@@ -63,7 +65,7 @@ def _stream(n, t_count, base, churn, seed):
     return snaps
 
 
-@pytest.mark.skipif(not HAVE_PCSR, reason="oracle/_ref/ref_pcsr.so not built (needs /root/reference)")
+@pytest.mark.skipif(not HAVE_PCSR, reason="oracle/_ref/ref_pcsr.so not built (oracle/build_ref.py needs the reference's sources)")
 @pytest.mark.parametrize("n,T,base,churn,seed", [(5, 4, 6, 3, 0), (16, 6, 60, 30, 1), (40, 5, 200, 200, 2), (120, 8, 900, 150, 3)])
 def test_pcsr_oracle_equals_reference_pcsr_on_random_streams(n, T, base, churn, seed):
     """Forward roll, then backward roll, like PCSRGraph (pcsr_graph.py:45-166); `churn == base` replaces every edge."""
@@ -94,102 +96,60 @@ def test_pcsr_oracle_equals_reference_pcsr_on_random_streams(n, T, base, churn, 
         ref.close()
 
 
-HAVE_KERNELS = os.path.exists(os.path.join(RE.REF_DIR, "gcn_f16.so"))
+@pytest.fixture(scope="module")
+def gl():
+    return np.load(os.path.join(GOLD, "ref_kernels_live.npz"))
 
 
-@pytest.mark.skipif(not (HAVE_CSR and HAVE_KERNELS), reason="oracle/_ref reference kernels not built")
+def _stored(gl, key):
+    """(row ids, rows) of one reference output kept in the fixture."""
+    return torch.from_numpy(gl[f"{key}/rows"]).long(), torch.from_numpy(gl[key])
+
+
 @pytest.mark.parametrize("case,feat,weighted", [("gcn_f16", 16, False), ("gcn_f100", 100, False), ("gcn_f128", 128, False),
                                                 ("gcnw_f7", 7, True)])
 @pytest.mark.parametrize("n,e,seed", [(12, 30, 0), (100, 1500, 1), (400, 6000, 2)])
-def test_aggregation_oracle_equals_reference_kernels_live(case, feat, weighted, n, e, seed):
+def test_aggregation_oracle_equals_reference_kernels_live(gl, case, feat, weighted, n, e, seed):
     """The CUDA kernels the reference's code generator emits for GCNConv (forward K0 on the in-edge CSR, backward K1 on
     the out-edge CSR), executed on the CPU by the SIMT shim with the reference's own launch geometry, against
-    oracle/aggregate.py on random graphs (a star around vertex 0 makes one long row and many short ones)."""
-    import torch
-
-    from oracle import aggregate as A
-
-    src, dst = _graph(n, e, seed)
-    star = np.arange(1, n, dtype=np.int32)
-    k = np.unique(np.concatenate([src.astype(np.int64) * n + dst, star.astype(np.int64) * n, star.astype(np.int64)]))
-    src, dst = (k // n).astype(np.int32), (k % n).astype(np.int32)
-    keep = src != dst
-    src, dst = src[keep], dst[keep]
-    ne = src.shape[0]
-    rng = np.random.default_rng(seed + 7)
-    w = rng.uniform(0.1, 1.0, size=ne).astype(np.float32)
-    fwd, bwd = RE.reference_static_graph(src, dst, w, n)
-    kernels, lib = RE.load_case(case)
-    norm = rng.uniform(0.2, 1.0, size=(n, 1)).astype(np.float32)
-    h = rng.standard_normal((n, feat)).astype(np.float32)
-    gin = rng.standard_normal((n, feat)).astype(np.float32)
-    tensors = {"Vhinb": h, "Vnormcen": norm, "Vnorminb": norm}
-    if weighted:
-        tensors["Vedge_weight"] = w.reshape(ne, 1).copy()
-    grads = [gin]
-    outs = {}
-    for kern in kernels:
-        for name, vt, shp in zip(kern["args"], kern["arg_types"], kern["arg_shapes"]):
-            if name not in tensors:
-                lead = ne if vt == "EDGE" else n
-                tensors[name] = np.zeros([lead] + shp, np.float32) if name in kern["rets"] else grads.pop(0)
-        csr = fwd if kern["parallel_mode"] == "DstParallel" else bwd
-        RE.run_reference_kernel(lib, kern, tensors, csr, n)
-        outs[kern["direction"]] = torch.from_numpy(tensors[kern["rets"][0]])
+    oracle/aggregate.py on random graphs (a star around vertex 0 makes one long row and many short ones).  The kernels'
+    outputs on these seeded inputs are stored in tests/golden/ref_kernels_live.npz (a seeded sample of rows)."""
+    src, dst, w, norm, h, gin = MG.live_gcn_inputs(feat, n, e, seed)
     f, b = S.forward_csr(src, dst, n), S.backward_csr(src, dst, n)
     ht, gt, nt = torch.from_numpy(h), torch.from_numpy(gin), torch.from_numpy(norm).reshape(-1)
     wt = torch.from_numpy(w) if weighted else None
     cols = 4 if feat == 7 else feat          # trap T1: for F=7 the reference launches 4 lanes per node
-    mine_f, mine_b = A.gcn_forward(f, ht, nt, wt), A.gcn_backward(b, gt, nt, wt)
-    A.assert_close_rel(mine_f[:, :cols], outs["forward"][:, :cols], rel=3e-6,
-                       abs_terms=A.gcn_forward(f, ht.abs(), nt, wt)[:, :cols], what=f"{case} forward")
-    A.assert_close_rel(mine_b[:, :cols], outs["backward"][:, :cols], rel=3e-6,
-                       abs_terms=A.gcn_backward(b, gt.abs(), nt, wt)[:, :cols], what=f"{case} backward")
-    if feat == 7:
-        assert torch.count_nonzero(outs["forward"][:, 4:]) == 0      # the columns the reference never writes
+    key = f"gcn/{case}/{n}_{e}_{seed}"
+    for direction, run in (("forward", A.gcn_forward), ("backward", A.gcn_backward)):
+        rows, ref = _stored(gl, f"{key}/{direction}")
+        csr, x = (f, ht) if direction == "forward" else (b, gt)
+        mine, mag = run(csr, x, nt, wt)[rows], run(csr, x.abs(), nt, wt)[rows]
+        A.assert_close_rel(mine[:, :cols], ref[:, :cols], rel=3e-6, abs_terms=mag[:, :cols], what=f"{case} {direction}")
+        if feat == 7 and direction == "forward":
+            assert torch.count_nonzero(ref[:, 4:]) == 0      # the columns the reference never writes
 
 
-@pytest.mark.skipif(not (HAVE_CSR and HAVE_KERNELS), reason="oracle/_ref reference kernels not built")
 @pytest.mark.parametrize("case,heads,dim", [("gat_h2d4", 2, 4), ("gat_h8d16", 8, 16)])
 @pytest.mark.parametrize("n,e,seed", [(30, 150, 0), (200, 2500, 1)])
-def test_stock_gat_oracle_equals_reference_kernels_live(case, heads, dim, n, e, seed):
-    """The three kernels the reference emits for GATConv as shipped (trap T2: a mean), forward and backward."""
-    import torch
-
-    from oracle import aggregate as A
-
-    src, dst = _graph(n, e, seed)
-    keep = src != dst
-    src, dst = src[keep], dst[keep]
-    ne = src.shape[0]
-    fwd, bwd = RE.reference_static_graph(src, dst, np.ones(ne, np.float32), n)
-    kernels, lib = RE.load_case(case)
-    rng = np.random.default_rng(seed + 11)
-    f32 = lambda *s: rng.standard_normal(s).astype(np.float32)
-    el, er, feat, gout = f32(n, heads, 1), f32(n, heads, 1), f32(n, heads, dim), f32(n, heads, dim)
-    tensors = {"Velinb": el, "Vercen": er, "Vfeat_srcinb": feat}
-    grads = [gout]
-    for kern in kernels:
-        for name, vt, shp in zip(kern["args"], kern["arg_types"], kern["arg_shapes"]):
-            if name not in tensors:
-                lead = ne if vt == "EDGE" else n
-                tensors[name] = np.zeros([lead] + shp, np.float32) if name in kern["rets"] else grads.pop(0)
-        RE.run_reference_kernel(lib, kern, tensors, fwd if kern["parallel_mode"] == "DstParallel" else bwd, n)
-    k0, k1, k2 = kernels
-    t = lambda name: torch.from_numpy(tensors[name])
+def test_stock_gat_oracle_equals_reference_kernels_live(gl, case, heads, dim, n, e, seed):
+    """The three kernels the reference emits for GATConv as shipped (trap T2: a mean), forward and backward; their
+    outputs on these seeded inputs are stored in tests/golden/ref_kernels_live.npz (a seeded sample of rows)."""
+    src, dst, el, er, feat, gout = MG.live_gat_inputs(heads, dim, n, e, seed)
+    t = torch.from_numpy
     f = S.forward_csr(src, dst, n)
-    out, o3, o4 = A.gat_stock_forward(f, t("Velinb"), t("Vercen"), t("Vfeat_srcinb"))
+    key = f"gat/{case}/{n}_{e}_{seed}"
     scale = lambda x: x.abs().mean() * torch.ones_like(x) + 1e-12
-    A.assert_close_rel(o3, t(k0["rets"][0]), rel=1e-6, abs_terms=scale(o3))
-    A.assert_close_rel(o4, t(k0["rets"][1]), rel=1e-6, abs_terms=scale(o4))
-    A.assert_close_rel(out, t(k1["rets"][0]), rel=3e-6, abs_terms=scale(out))
-    d_feat, d_el, d_er, m_feat, m_el, m_er = A.gat_stock_backward(f, t("Velinb"), t("Vercen"), t("Vfeat_srcinb"),
-                                                                  torch.from_numpy(gout), return_mag=True)
-    rets = [t(r) for r in k2["rets"]]
-    ref_dfeat = [r for r in rets if r.shape[-1] == dim and r.dim() == 3 and r.shape[1] == heads][0] if dim != 1 else rets[0]
-    small = [r for r in rets if r.shape[-1] == 1]
-    A.assert_close_rel(d_feat, ref_dfeat, rel=5e-6, abs_terms=scale(ref_dfeat), what="d_feat")
-    ref_der = min(small, key=lambda x: float(x.abs().max()))
-    ref_del = max(small, key=lambda x: float(x.abs().max()))
-    A.assert_close_rel(d_el, ref_del, rel=2e-5, abs_terms=m_el, what="d_el")
-    A.assert_close_rel(d_er, ref_der, rel=2e-5, abs_terms=m_er, what="d_er")
+
+    def check(role, mine, rel, abs_terms, what=""):
+        rows, ref = _stored(gl, f"{key}/{role}")
+        A.assert_close_rel(mine[rows], ref.reshape((-1,) + tuple(mine.shape[1:])), rel=rel, abs_terms=abs_terms[rows], what=what)
+
+    out, o3, o4 = A.gat_stock_forward(f, t(el), t(er), t(feat))
+    check("v3", o3, 1e-6, scale(o3))
+    check("v4", o4, 1e-6, scale(o4))
+    check("out", out, 3e-6, scale(out))
+    d_feat, d_el, d_er, m_feat, m_el, m_er = A.gat_stock_backward(f, t(el), t(er), t(feat), t(gout), return_mag=True)
+    ref_dfeat_scale = float(gl[f"{key}/d_feat_abs_mean"]) * torch.ones_like(d_feat) + 1e-12
+    check("d_feat", d_feat, 5e-6, ref_dfeat_scale, what="d_feat")
+    check("d_el", d_el, 2e-5, m_el, what="d_el")
+    check("d_er", d_er, 2e-5, m_er, what="d_er")
