@@ -13,17 +13,21 @@ class _EdgeDot(torch.autograd.Function):
     @staticmethod
     def forward(ctx, z, a, b):
         z = z.contiguous()
+        ctx.save_for_backward(z, a, b)
+        if z.shape[1] == 0:             # every dot product is empty: zero scores, zero gradient (as torch computes them)
+            return torch.zeros(a.shape[0], dtype=torch.float32, device=z.device)
         out = torch.empty(a.shape[0], dtype=torch.float32, device=z.device)
         _lib.call("stg_edge_dot_f32", z.data_ptr(), z.shape[1], a.data_ptr(), b.data_ptr(), a.shape[0], out.data_ptr(),
                   _lib.current_stream_ptr())
         kernels.launch_count += 1
-        ctx.save_for_backward(z, a, b)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         z, a, b = ctx.saved_tensors
         d_z = torch.zeros_like(z)
+        if z.shape[1] == 0:
+            return d_z, None, None
         _lib.call("stg_edge_dot_bwd_f32", z.data_ptr(), z.shape[1], a.data_ptr(), b.data_ptr(), a.shape[0],
                   grad_out.contiguous().data_ptr(), d_z.data_ptr(), _lib.current_stream_ptr())
         kernels.launch_count += 1
