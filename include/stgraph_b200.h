@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define STG_ABI_VERSION 3
+#define STG_ABI_VERSION 4
 
 typedef enum StgStatus {
   STG_OK = 0,
@@ -112,6 +112,17 @@ int stg_agg_packed_sum_f32(const StgCsrView* g, const StgEdgeMeta* meta, const f
 int stg_agg_packed_sum_strided_f32(const StgCsrView* g, const StgEdgeMeta* meta, const float* x, int32_t feat,
                                    int32_t x_ld, const float* row_scale, float* out, int32_t out_ld,
                                    int32_t accumulate, void* stream);
+
+/* 16-bit feature rows (torch.autocast): x and out are [num_nodes, feat] row-major bf16, or both fp16, as `dtype` says.
+ * The scales and the packed records stay fp32; every product and the running sum are fp32, and each output element is
+ * rounded to the 16-bit type once.  Assign mode only.  A graph's packed array (stg_csr_pack_edge_meta_f32) serves the
+ * fp32 and the 16-bit entry points alike, and the packed sums equal the plain ones bit for bit.  feat == 0 is a no-op. */
+typedef enum StgDtype { STG_DTYPE_BF16 = 1, STG_DTYPE_F16 = 2 } StgDtype;
+int stg_agg_scaled_sum_h16(const StgCsrView* g, const void* x, int32_t feat, int32_t dtype,
+                           const float* nbr_scale, const float* edge_scale, const float* row_scale,
+                           void* out, void* stream);
+int stg_agg_packed_sum_h16(const StgCsrView* g, const StgEdgeMeta* meta, const void* x, int32_t feat,
+                           int32_t dtype, const float* row_scale, void* out, void* stream);
 
 /* Accumulating form: out[r,:] += row_scale[r] * sum(...).  Used when a row's edge set is split in two CSRs
  * (edges to locally owned sources / edges to halo sources) so that the first pass overlaps the halo

@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STG_B200_LIB") or os.path.join(_HERE, "lib", "libstgraph_b200.so")   # env: A/B builds only
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 VM_MAX_TENSORS = 24
 VM_MAX_INSTR = 96
 VM_MAX_REGS = 48
@@ -95,6 +95,10 @@ _SIGNATURES = {
                                               c_void_p], True),
     "stg_agg_packed_sum_strided_f32": (ctypes.c_int, [_P(StgCsrView), c_void_p, c_void_p, c_int32, c_int32, c_void_p,
                                                       c_void_p, c_int32, c_int32, c_void_p], True),
+    "stg_agg_scaled_sum_h16": (ctypes.c_int, [_P(StgCsrView), c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                              c_void_p, c_void_p], True),
+    "stg_agg_packed_sum_h16": (ctypes.c_int, [_P(StgCsrView), c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p,
+                                              c_void_p], True),
     "stg_halo_push_f32": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int64, _P(c_void_p), c_int32,
                                          c_int32, c_void_p], True),
     "stg_agg_packed_sum_rows_f32": (ctypes.c_int, [_P(StgCsrView), c_void_p, c_void_p, c_void_p, c_int32, c_void_p,

@@ -172,14 +172,14 @@ class Executor:
         self.ts.clear_current_tensor_state()
         return ret
 
-    def _alloc(self, var, zero, like_map):
+    def _alloc(self, var, zero, like_map, dtype=None):
         lead = self.num_edges if var.is_edgevar() else self.num_nodes
         size = [lead] + list(var.var_shape)
         fn = self.new_zeros if (zero or self.new_empty is None) else self.new_empty
         dev = var.device
         if dev is None or (isinstance(dev, torch.device) and dev.type != "cuda"):
             dev = next(iter(like_map.values())).device
-        return fn(size=size, dtype=var.var_dtype, device=dev, requires_grad=False)
+        return fn(size=size, dtype=var.var_dtype if dtype is None else dtype, device=dev, requires_grad=False)
 
     def _alloc_unit_outputs(self, unit, tensor_map):
         needs_zero = set()
@@ -187,6 +187,12 @@ class Executor:
         for la in unit.launches:
             needs_zero |= la.needs_zero
             written |= set(la.writes)
+            # A scaled sum over bf16 / fp16 rows writes rows of that type.  The traced program cannot say so: it types
+            # ``h * norm`` by promotion (fp32) and a gradient by its first operand, so the output takes x's dtype here.
+            if la.kind == "scaled_sum" and la.out.id not in tensor_map:
+                x = tensor_map.get(la.x.id)
+                if x is not None and x.dtype in kernels.H16_DTYPES:
+                    tensor_map[la.out.id] = self._alloc(la.out, False, tensor_map, dtype=x.dtype)
         for var in unit.unit_rets():
             if var.id not in tensor_map:
                 tensor_map[var.id] = self._alloc(var, var in needs_zero or var not in written, tensor_map)

@@ -940,17 +940,6 @@ int agg_scaled_sum_device(const StgCsrView* g, const float* x, int32_t feat, con
 
 using namespace stg;
 
-static int validate_view(const StgCsrView* g, bool need_eids) {
-  STG_CHECK_ARG(g != nullptr, "graph view is NULL");
-  STG_CHECK_ARG(g->num_nodes >= 0 && g->num_edges >= 0, "negative graph size (%d nodes, %d edges)",
-                g->num_nodes, g->num_edges);
-  STG_CHECK_ARG(g->row_offset != nullptr, "row_offset is NULL");
-  STG_CHECK_ARG(g->num_edges == 0 || g->column_indices != nullptr, "column_indices is NULL");
-  STG_CHECK_ARG(!need_eids || g->eids_identity || g->num_edges == 0 || g->eids != nullptr,
-                "eids is NULL but an edge tensor is indexed by edge id");
-  return STG_OK;
-}
-
 STG_API int stg_agg_scaled_sum_f32(const StgCsrView* g, const float* x, int32_t feat,
                                       const float* nbr_scale, const float* edge_scale,
                                       const float* row_scale, float* out, void* stream) {

@@ -48,6 +48,18 @@ inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Checks every aggregation entry point makes on a CSR view before it launches anything.
+inline int validate_view(const StgCsrView* g, bool need_eids) {
+  STG_CHECK_ARG(g != nullptr, "graph view is NULL");
+  STG_CHECK_ARG(g->num_nodes >= 0 && g->num_edges >= 0, "negative graph size (%d nodes, %d edges)",
+                g->num_nodes, g->num_edges);
+  STG_CHECK_ARG(g->row_offset != nullptr, "row_offset is NULL");
+  STG_CHECK_ARG(g->num_edges == 0 || g->column_indices != nullptr, "column_indices is NULL");
+  STG_CHECK_ARG(!need_eids || g->eids_identity || g->num_edges == 0 || g->eids != nullptr,
+                "eids is NULL but an edge tensor is indexed by edge id");
+  return STG_OK;
+}
+
 // Number of SMs of the current device (cached per process; 148 on B200).
 int sm_count();
 

@@ -27,6 +27,60 @@ def _check(t: torch.Tensor, name: str, dtype=torch.float32):
     return t
 
 
+#: 16-bit feature types of the aggregation (``StgDtype``): fp32 accumulation, one rounding per output element
+H16_DTYPES = {torch.bfloat16: 1, torch.float16: 2}
+
+
+def _agg_h16(view, meta, x, nbr_scale, edge_scale, row_scale, out, accumulate, stream, out_rows=None):
+    """16-bit ``x`` (``stg_agg_scaled_sum_h16`` / ``stg_agg_packed_sum_h16``): contiguous, assign-only, ``out`` of ``x``'s
+    dtype; the scales stay fp32.  Everything is checked before the launch."""
+    global launch_count
+    if accumulate is not False:
+        raise ValueError(f"accumulate={accumulate!r} is an fp32-only form of the aggregation; {x.dtype} x is assign-only")
+    if out_rows is not None:
+        raise ValueError(f"out_rows is an fp32-only form of the aggregation (got {x.dtype} x)")
+    for nm, t in (("x", x), ("out", out)):
+        if isinstance(t, torch.Tensor) and not t.is_contiguous():
+            raise ValueError(f"padded / strided rows are an fp32-only form of the aggregation: {x.dtype} {nm} must be contiguous")
+    _check(x, "x", x.dtype)
+    if x.dim() < 2:
+        raise ValueError("x must be [rows, feat...]")
+    n = view.num_nodes
+    feat = x.numel() // max(x.shape[0], 1)
+    for nm, t in (("nbr_scale", nbr_scale), ("edge_scale", edge_scale), ("row_scale", row_scale)):
+        if t is not None:
+            _check(t, nm)
+    if nbr_scale is not None and nbr_scale.numel() != x.shape[0]:
+        raise ValueError(f"nbr_scale must have one entry per row of x ({x.shape[0]}), got {nbr_scale.numel()}")
+    if row_scale is not None and row_scale.numel() != n:
+        raise ValueError(f"row_scale must have {n} elements, got {row_scale.numel()}")
+    if edge_scale is not None and edge_scale.numel() < view.num_edges:
+        raise ValueError(f"edge_scale has {edge_scale.numel()} elements for {view.num_edges} edges")
+    if meta is not None:
+        _check(meta, "meta", torch.int32)
+        if meta.numel() < 2 * view.num_edges:
+            raise ValueError(f"meta has {meta.numel() // 2} entries for {view.num_edges} edges")
+    if out is None:
+        if x.shape[0] != n:
+            raise ValueError(f"x has {x.shape[0]} rows for a view of {n} rows: pass out= for a row slice")
+        out = torch.empty_like(x)
+    else:
+        _check(out, "out", x.dtype)
+        if out.shape[0] != n or out.numel() != n * feat:
+            raise ValueError(f"out must be [{n}, {feat}], got {tuple(out.shape)}")
+    if n == 0 or feat == 0:
+        return out
+    st = stream if stream is not None else _lib.current_stream_ptr()
+    if meta is None:
+        _lib.call("stg_agg_scaled_sum_h16", ctypes.byref(view), x.data_ptr(), feat, H16_DTYPES[x.dtype], _lib.ptr(nbr_scale),
+                  _lib.ptr(edge_scale), _lib.ptr(row_scale), out.data_ptr(), st)
+    else:
+        _lib.call("stg_agg_packed_sum_h16", ctypes.byref(view), meta.data_ptr(), x.data_ptr(), feat, H16_DTYPES[x.dtype],
+                  _lib.ptr(row_scale), out.data_ptr(), st)
+    launch_count += 1 + (1 if view.hub_threshold > 0 else 0)
+    return out
+
+
 def agg_scaled_sum(view: _lib.StgCsrView, x: torch.Tensor, nbr_scale=None, edge_scale=None, row_scale=None,
                    out: torch.Tensor | None = None, accumulate=False, stream=None, out_rows=None) -> torch.Tensor:
     """``out[r] = row_scale[r] * sum_e nbr_scale[c_e] * edge_scale[eid_e] * x[c_e]`` (see ``stg_agg_scaled_sum_f32``).
@@ -34,8 +88,13 @@ def agg_scaled_sum(view: _lib.StgCsrView, x: torch.Tensor, nbr_scale=None, edge_
     ``accumulate``: False (assign), True (``+=``) or ``"red"`` (``red.global.add``).  ``out_rows`` (int32, strictly
     increasing): the view holds a subset of the output rows, view row ``i`` is ``out[out_rows[i]]``
     (``stg_agg_scaled_sum_rows_f32``); ``out`` is then required.
+
+    A bf16 / fp16 ``x`` is summed in fp32 and ``out`` has ``x``'s dtype (``stg_agg_scaled_sum_h16``); that form is
+    contiguous and assign-only, and the scales stay fp32.
     """
     global launch_count
+    if isinstance(x, torch.Tensor) and x.dtype in H16_DTYPES:
+        return _agg_h16(view, None, x, nbr_scale, edge_scale, row_scale, out, accumulate, stream, out_rows)
     _check(x, "x")
     n = view.num_nodes                      # rows of this view (a row slice of a partitioned graph has fewer rows than x)
     if out_rows is not None:
@@ -134,8 +193,11 @@ def agg_packed_sum(view: _lib.StgCsrView, meta: torch.Tensor, x: torch.Tensor, r
                    out: torch.Tensor | None = None, accumulate=False, stream=None) -> torch.Tensor:
     """``out[r] = row_scale[r] * sum_e meta[e].scale * x[meta[e].col]`` (``stg_agg_packed_sum_strided_f32``): the sums
     of :func:`agg_scaled_sum`, bit for bit, with one coalesced 8-byte load per edge instead of dependent gathers.
-    ``x`` / ``out`` may be row-padded 2-D views (:func:`padded_rows`)."""
+    ``x`` / ``out`` may be row-padded 2-D views (:func:`padded_rows`).  A bf16 / fp16 ``x`` takes the 16-bit form of
+    :func:`agg_scaled_sum` (``stg_agg_packed_sum_h16``: contiguous, assign-only) with the same ``meta``."""
     global launch_count
+    if isinstance(x, torch.Tensor) and x.dtype in H16_DTYPES:
+        return _agg_h16(view, meta, x, None, None, row_scale, out, accumulate, stream)
     x_ld = _row_stride(x, "x")
     _check(meta, "meta", torch.int32)
     n = view.num_nodes

@@ -234,9 +234,10 @@ def sliding_window_snapshots(src, dst, base: int, slide: int, num_snapshots: int
     return snaps
 
 
-def gcn_algorithmic_bytes(num_nodes: int, num_edges: int, feat: int, weighted: bool = False) -> int:
-    """Compulsory traffic of one fused aggregation launch (SURVEY.md section 8(d))."""
-    b = 4 * (2 * num_nodes * feat + num_edges + (num_nodes + 1) + 2 * num_nodes)
+def gcn_algorithmic_bytes(num_nodes: int, num_edges: int, feat: int, weighted: bool = False, elem_bytes: int = 4) -> int:
+    """Compulsory traffic of one fused aggregation launch (SURVEY.md section 8(d)); ``elem_bytes`` is the size of one
+    element of the feature rows read and written (2 for bf16 / fp16 rows; indices and scales stay 4 bytes)."""
+    b = elem_bytes * 2 * num_nodes * feat + 4 * (num_edges + (num_nodes + 1) + 2 * num_nodes)
     if weighted:
         b += 4 * num_edges
     return b
