@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define STG_ABI_VERSION 4
+#define STG_ABI_VERSION 5
 
 typedef enum StgStatus {
   STG_OK = 0,
@@ -241,6 +241,19 @@ int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_out,
                             int32_t heads, int32_t dim, float slope,
                             float* d_feat, float* d_el, float* d_er,
                             float* dot_scratch, void* stream);
+/* 16-bit form of the two above (torch.autocast): feat and d_feat are [N,H,D] bf16, or both fp16, as `dtype`
+ * (StgDtype) says; el, er, out, grad_out, row_max, row_sum, d_el, d_er and dot_scratch stay fp32.  An element of feat is
+ * widened to fp32 when it is loaded and d_feat is rounded to nearest even once, when it is stored.  The lanes are laid
+ * out as in the fp32 entry points (4 elements per lane when dim % 4 == 0, feat / d_feat are 8-byte and out / grad_out
+ * 16-byte aligned; otherwise 1), so the results equal those of the fp32 entry points on the widened feat bit for bit,
+ * and d_feat equals their d_feat rounded to the 16-bit type. */
+int stg_gat_softmax_fwd_h16(const StgCsrView* g_in, const float* el, const float* er, const void* feat,
+                            int32_t heads, int32_t dim, int32_t dtype, float slope,
+                            float* out, float* row_max, float* row_sum, void* stream);
+int stg_gat_softmax_bwd_h16(const StgCsrView* g_in, const StgCsrView* g_out, const float* el, const float* er,
+                            const void* feat, const float* out, const float* grad_out, const float* row_max,
+                            const float* row_sum, int32_t heads, int32_t dim, int32_t dtype, float slope,
+                            void* d_feat, float* d_el, float* d_er, float* dot_scratch, void* stream);
 
 /* ------------------------------------------- generic fused vertex program */
 /* A lowered execution unit: straight-line register code evaluated per

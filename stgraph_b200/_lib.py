@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STG_B200_LIB") or os.path.join(_HERE, "lib", "libstgraph_b200.so")   # env: A/B builds only
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 VM_MAX_TENSORS = 24
 VM_MAX_INSTR = 96
 VM_MAX_REGS = 48
@@ -121,6 +121,11 @@ _SIGNATURES = {
                                                c_float, c_void_p, c_void_p, c_void_p, c_void_p], True),
     "stg_gat_softmax_bwd_f32": (ctypes.c_int, [_P(StgCsrView), _P(StgCsrView), c_void_p, c_void_p, c_void_p,
                                                c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_float,
+                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p], True),
+    "stg_gat_softmax_fwd_h16": (ctypes.c_int, [_P(StgCsrView), c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32,
+                                               c_float, c_void_p, c_void_p, c_void_p, c_void_p], True),
+    "stg_gat_softmax_bwd_h16": (ctypes.c_int, [_P(StgCsrView), _P(StgCsrView), c_void_p, c_void_p, c_void_p,
+                                               c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_float,
                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p], True),
     "stg_vm_run_f32": (ctypes.c_int, [_P(StgCsrView), _P(StgVmProgram), _P(c_void_p), c_void_p], True),
     "stg_edge_dot_f32": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_void_p, c_void_p], True),

@@ -21,6 +21,7 @@
 // HBM-roofline kernels; algorithmic bytes: fwd 4*(2*N*H*D + 4*N*H + E + N+1),
 // bwd 4*(4*N*H*D + 6*N*H + 2*(E+N+1)).
 #include "common.cuh"
+#include "h16.cuh"
 
 #include <cooperative_groups.h>
 
@@ -44,6 +45,49 @@ __device__ __forceinline__ void stv(float* p, typename VecT<VEC>::type v) {
   using T = typename VecT<VEC>::type;
   *reinterpret_cast<T*>(p) = v;
 }
+// feat / d_feat elements of storage type FT (float, __nv_bfloat16, __half): VEC of them per lane, one 8- or 2-byte
+// access for 16-bit rows, widened to fp32 and rounded to nearest even on the store.  The forward edge loop keeps a
+// gathered row in its loaded form (FtRaw) until the batch's arithmetic: widening right after the load, inside the
+// `if (L.act[k])` of the batch, made the compiler branch around each load and wait for it before issuing the next one
+// (config 3: 0.194 ms against 0.152 ms for fp32 rows).  Backward pass A widens on load: it was not slower that way, and
+// with the later widening its d_er no longer matched the fp32 kernel's bit for bit.
+template <int VEC, typename FT> struct FtRaw { using type = typename Raw<VEC>::type; };
+template <int VEC> struct FtRaw<VEC, float> { using type = typename VecT<VEC>::type; };
+using stg::zero_vec;
+__device__ __forceinline__ void zero_vec(uint2& a) { a = make_uint2(0u, 0u); }
+__device__ __forceinline__ void zero_vec(unsigned short& a) { a = 0; }
+
+template <int VEC, typename FT>
+__device__ __forceinline__ typename FtRaw<VEC, FT>::type ldraw(const FT* p) {
+  if constexpr (std::is_same_v<FT, float>) return ldv<VEC>(p);
+  else return __ldg(reinterpret_cast<const typename Raw<VEC>::type*>(p));
+}
+template <int VEC, typename FT>
+__device__ __forceinline__ typename VecT<VEC>::type widen(const typename FtRaw<VEC, FT>::type& r) {
+  if constexpr (std::is_same_v<FT, float>) {
+    return r;
+  } else {
+    float f[VEC];
+    unpack<FT, VEC>(r, f);
+    if constexpr (VEC == 4) return make_float4(f[0], f[1], f[2], f[3]);
+    else return f[0];
+  }
+}
+template <int VEC, typename FT>
+__device__ __forceinline__ typename VecT<VEC>::type ldf(const FT* p) {
+  return widen<VEC, FT>(ldraw<VEC>(p));
+}
+template <int VEC, typename FT>
+__device__ __forceinline__ void stf(FT* p, typename VecT<VEC>::type v) {
+  if constexpr (std::is_same_v<FT, float>) {
+    stv<VEC>(p, v);
+  } else {
+    float f[VEC];
+    if constexpr (VEC == 4) f[0] = v.x, f[1] = v.y, f[2] = v.z, f[3] = v.w;
+    else f[0] = v;
+    *reinterpret_cast<typename Raw<VEC>::type*>(p) = pack<FT, VEC>(f);
+  }
+}
 __device__ __forceinline__ float dotv(float a, float b) { return a * b; }
 __device__ __forceinline__ float dotv(float2 a, float2 b) { return a.x * b.x + a.y * b.y; }
 __device__ __forceinline__ float dotv(float4 a, float4 b) { return a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w; }
@@ -58,7 +102,10 @@ __device__ __forceinline__ float4 shfl_xor_t(unsigned m, float4 v, int o) {
                      __shfl_xor_sync(m, v.w, o));
 }
 
+// FT: storage type of feat and d_feat; every other tensor, and all arithmetic, is fp32.
+template <typename FT>
 struct GatParams {
+  using feat_t = FT;
   const int32_t* __restrict__ row_off;
   const int32_t* __restrict__ col;
   const int32_t* __restrict__ hub_rows;
@@ -71,13 +118,13 @@ struct GatParams {
   float slope;
   const float* __restrict__ el;     // [N,H]
   const float* __restrict__ er;     // [N,H]
-  const float* __restrict__ feat;   // [N,H,D]
+  const FT* __restrict__ feat;      // [N,H,D]
   const float* __restrict__ out;    // [N,H,D]  (backward)
   const float* __restrict__ gout;   // [N,H,D]  (backward)
   float* __restrict__ row_max;      // [N,H]
   float* __restrict__ row_sum;      // [N,H]
   float* __restrict__ dot;          // [N,H]    (backward scratch)
-  float* __restrict__ o_vec;        // forward: out; backward pass B: d_feat
+  float* __restrict__ o_vec;        // forward: out; backward pass B: d_feat (FT elements, see gat_bwd_store)
   float* __restrict__ o_head;       // backward: d_er (pass A) / d_el (pass B)
 };
 
@@ -87,7 +134,8 @@ struct Lanes {
   unsigned gmask;
   int off[NACC], hk[NACC];
   bool act[NACC];
-  __device__ __forceinline__ void init(const GatParams& p) {
+  template <class P>
+  __device__ __forceinline__ void init(const P& p) {
     const int lane = threadIdx.x & 31;
     gl = lane & (GROUP - 1);
     gmask = (GROUP == 32) ? 0xffffffffu : (((1u << GROUP) - 1u) << (lane & ~(GROUP - 1)));
@@ -158,11 +206,11 @@ struct FwdState {
   }
 };
 
-template <int VEC, int GROUP, int NACC>
-__device__ __forceinline__ void gat_fwd_edges(const GatParams& p, const Lanes<VEC, GROUP, NACC>& L, int row, int beg,
+template <int VEC, int GROUP, int NACC, class P>
+__device__ __forceinline__ void gat_fwd_edges(const P& p, const Lanes<VEC, GROUP, NACC>& L, int row, int beg,
                                               int end, int first_batch, int batch_step,
                                               FwdState<VEC, GROUP, NACC>& st, int nx_c) {
-  using T = typename VecT<VEC>::type;
+  using FT = typename P::feat_t;
   constexpr int U = UnrollFor<NACC>::value;
   float erk[NACC];
 #pragma unroll
@@ -181,7 +229,7 @@ __device__ __forceinline__ void gat_fwd_edges(const GatParams& p, const Lanes<VE
     auto group = [&](auto uu, int j) {
       constexpr int UU = decltype(uu)::value;
       float sc[UU][NACC];
-      T v[UU][NACC];
+      typename FtRaw<VEC, FT>::type v[UU][NACC];
 #pragma unroll
       for (int u = 0; u < UU; ++u) {
         const int c = __shfl_sync(L.gmask, my_c, j + u, GROUP);
@@ -191,7 +239,7 @@ __device__ __forceinline__ void gat_fwd_edges(const GatParams& p, const Lanes<VE
           zero_vec(v[u][k]);
           if (L.act[k]) {
             sc[u][k] = lrelu(__ldg(p.el + static_cast<size_t>(c) * p.heads + L.hk[k]) + erk[k], p.slope);
-            v[u][k] = ldv<VEC>(p.feat + static_cast<size_t>(c) * p.hd + L.off[k]);
+            v[u][k] = ldraw<VEC>(p.feat + static_cast<size_t>(c) * p.hd + L.off[k]);
           }
         }
       }
@@ -211,7 +259,7 @@ __device__ __forceinline__ void gat_fwd_edges(const GatParams& p, const Lanes<VE
         for (int u = 0; u < UU; ++u) {
           const float pe = __expf(sc[u][k] - st.m[k]);
           st.s[k] += pe;
-          fma_vec(st.acc[k], pe, v[u][k]);
+          fma_vec(st.acc[k], pe, widen<VEC, FT>(v[u][k]));
         }
       }
     };
@@ -220,14 +268,14 @@ __device__ __forceinline__ void gat_fwd_edges(const GatParams& p, const Lanes<VE
 }
 
 // columns of the first batch a lane group visits (the pipelined kernels load them one row ahead instead)
-template <int GROUP>
-__device__ __forceinline__ int first_cols(const GatParams& p, int beg, int end, int first_batch, int gl) {
+template <int GROUP, class P>
+__device__ __forceinline__ int first_cols(const P& p, int beg, int end, int first_batch, int gl) {
   const int e = beg + first_batch * GROUP + gl;
   return (e < end) ? ld_stream(p.col + e) : 0;
 }
 
-template <int VEC, int GROUP, int NACC>
-__device__ __forceinline__ void gat_fwd_store(const GatParams& p, const Lanes<VEC, GROUP, NACC>& L, int row,
+template <int VEC, int GROUP, int NACC, class P>
+__device__ __forceinline__ void gat_fwd_store(const P& p, const Lanes<VEC, GROUP, NACC>& L, int row,
                                               bool nonempty, FwdState<VEC, GROUP, NACC>& st) {
 #pragma unroll
   for (int k = 0; k < NACC; ++k) {
@@ -242,8 +290,8 @@ __device__ __forceinline__ void gat_fwd_store(const GatParams& p, const Lanes<VE
   }
 }
 
-template <int VEC, int GROUP, int NACC>
-__global__ void __launch_bounds__(kGatThreads) gat_fwd_kernel(const GatParams p) {
+template <typename FT, int VEC, int GROUP, int NACC>
+__global__ void __launch_bounds__(kGatThreads) gat_fwd_kernel(const GatParams<FT> p) {
   Lanes<VEC, GROUP, NACC> L;
   L.init(p);
   const int warp = blockIdx.x * (kGatThreads / 32) + (threadIdx.x >> 5);
@@ -270,8 +318,8 @@ struct BwdState {
   float acch[NACC], c_a[NACC], c_m[NACC], c_inv[NACC], c_dot[NACC];
 };
 
-template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL>
-__device__ __forceinline__ void gat_bwd_prologue(const GatParams& p, const Lanes<VEC, GROUP, NACC>& L, int row,
+template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL, class P>
+__device__ __forceinline__ void gat_bwd_prologue(const P& p, const Lanes<VEC, GROUP, NACC>& L, int row,
                                                  BwdState<VEC, GROUP, NACC>& st, bool write_dot) {
   const size_t rh = static_cast<size_t>(row) * p.heads;
 #pragma unroll
@@ -284,7 +332,7 @@ __device__ __forceinline__ void gat_bwd_prologue(const GatParams& p, const Lanes
     const size_t ro = static_cast<size_t>(row) * p.hd + L.off[k];
     if (L.act[k]) {
       if (SRC_PARALLEL) {
-        st.cen[k] = ldv<VEC>(p.feat + ro);
+        st.cen[k] = ldf<VEC>(p.feat + ro);
         st.c_a[k] = __ldg(p.el + rh + L.hk[k]);
       } else {
         st.cen[k] = ldv<VEC>(p.gout + ro);
@@ -302,8 +350,8 @@ __device__ __forceinline__ void gat_bwd_prologue(const GatParams& p, const Lanes
   }
 }
 
-template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL>
-__device__ __forceinline__ void gat_bwd_edges(const GatParams& p, const Lanes<VEC, GROUP, NACC>& L, int beg, int end,
+template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL, class P>
+__device__ __forceinline__ void gat_bwd_edges(const P& p, const Lanes<VEC, GROUP, NACC>& L, int beg, int end,
                                               int first_batch, int batch_step, BwdState<VEC, GROUP, NACC>& st,
                                               int nx_c) {
   using T = typename VecT<VEC>::type;
@@ -337,7 +385,7 @@ __device__ __forceinline__ void gat_bwd_edges(const GatParams& p, const Lanes<VE
               inv[u][k] = sv > 0.f ? 1.f / sv : 0.f;
               dt[u][k] = __ldg(p.dot + ch + L.hk[k]);
             } else {                 // neighbour = source: its el and feature row
-              nb[u][k] = ldv<VEC>(p.feat + static_cast<size_t>(c) * p.hd + L.off[k]);
+              nb[u][k] = ldf<VEC>(p.feat + static_cast<size_t>(c) * p.hd + L.off[k]);
               pre[u][k] = __ldg(p.el + ch + L.hk[k]) + st.c_a[k];
               mm[u][k] = st.c_m[k];
               inv[u][k] = st.c_inv[k];
@@ -365,20 +413,23 @@ __device__ __forceinline__ void gat_bwd_edges(const GatParams& p, const Lanes<VE
   }
 }
 
-template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL>
-__device__ __forceinline__ void gat_bwd_store(const GatParams& p, const Lanes<VEC, GROUP, NACC>& L, int row,
+template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL, class P>
+__device__ __forceinline__ void gat_bwd_store(const P& p, const Lanes<VEC, GROUP, NACC>& L, int row,
                                               BwdState<VEC, GROUP, NACC>& st) {
   const size_t rh = static_cast<size_t>(row) * p.heads;
 #pragma unroll
   for (int k = 0; k < NACC; ++k) {
     if (!L.act[k]) continue;
-    if (SRC_PARALLEL) stv<VEC>(p.o_vec + static_cast<size_t>(row) * p.hd + L.off[k], st.accv[k]);
+    if (SRC_PARALLEL) {
+      using FT = typename P::feat_t;
+      stf<VEC>(reinterpret_cast<FT*>(p.o_vec) + static_cast<size_t>(row) * p.hd + L.off[k], st.accv[k]);
+    }
     if (L.off[k] % p.dim == 0) p.o_head[rh + L.hk[k]] = st.acch[k];
   }
 }
 
-template <int VEC, int GROUP, int NACC, bool SRC_PARALLEL>
-__global__ void __launch_bounds__(kGatThreads) gat_bwd_kernel(const GatParams p) {
+template <typename FT, int VEC, int GROUP, int NACC, bool SRC_PARALLEL>
+__global__ void __launch_bounds__(kGatThreads) gat_bwd_kernel(const GatParams<FT> p) {
   Lanes<VEC, GROUP, NACC> L;
   L.init(p);
   const int warp = blockIdx.x * (kGatThreads / 32) + (threadIdx.x >> 5);
@@ -411,9 +462,9 @@ constexpr int kGatGiantEdges = 1024;
 
 template <int NACC> struct HubThreads { static constexpr int value = NACC >= 4 ? kGatHubThreads / 2 : kGatHubThreads; };
 
-template <int VEC, int GROUP, int NACC, int KIND>
+template <typename FT, int VEC, int GROUP, int NACC, int KIND>
 __global__ void __cluster_dims__(kGatCluster, 1, 1) __launch_bounds__(HubThreads<NACC>::value, NACC == 1 ? 4 : 1)
-    gat_hub_kernel(const GatParams p) {
+    gat_hub_kernel(const GatParams<FT> p) {
   using T = typename VecT<VEC>::type;
   namespace cg = cooperative_groups;
   constexpr int WARPS = HubThreads<NACC>::value / 32;
@@ -564,8 +615,8 @@ constexpr int kGatRowsPerWarp = 16;
 // GQ: global row queue as in agg.cu (persistent grid, warps draw chunks of rows_per_block rows from the view's device
 // counter; the last block rearms it): config 3 has 1323 blocks of 128 rows on 592 block slots, i.e. 2.2 waves whose
 // last one is a third full -- with the queue every warp stays busy until the rows run out.
-template <int VEC, int NACC, int KIND, bool GQ = false>
-__global__ void __launch_bounds__(kGatThreads, NACC == 1 ? 4 : 1) gat_rows_pipe_kernel(const GatParams p, int rows_per_block) {
+template <typename FT, int VEC, int NACC, int KIND, bool GQ = false>
+__global__ void __launch_bounds__(kGatThreads, NACC == 1 ? 4 : 1) gat_rows_pipe_kernel(const GatParams<FT> p, int rows_per_block) {
   constexpr int GROUP = 32;
   __shared__ int next_row;
   Lanes<VEC, GROUP, NACC> L;
@@ -673,8 +724,8 @@ inline int gat_hub_grid_mult() {
   return v;
 }
 
-template <int VEC, int GROUP, int NACC>
-int launch_gat(const GatParams& p, int which, cudaStream_t s) {
+template <typename FT, int VEC, int GROUP, int NACC>
+int launch_gat(const GatParams<FT>& p, int which, cudaStream_t s) {
   const int rows_per_block = (kGatThreads / 32) * (32 / GROUP);
   const int blocks = (p.num_rows + rows_per_block - 1) / rows_per_block;
   if (blocks <= 0) return STG_OK;
@@ -683,9 +734,9 @@ int launch_gat(const GatParams& p, int which, cudaStream_t s) {
   // Hub rows first: the longest rows are the critical path, the row kernel fills the SMs they leave idle.
   if (hubs) {
     constexpr int ht = HubThreads<NACC>::value;
-    if (which == 0) gat_hub_kernel<VEC, GROUP, NACC, 0><<<hub_grid, ht, 0, s>>>(p);
-    else if (which == 1) gat_hub_kernel<VEC, GROUP, NACC, 1><<<hub_grid, ht, 0, s>>>(p);
-    else gat_hub_kernel<VEC, GROUP, NACC, 2><<<hub_grid, ht, 0, s>>>(p);
+    if (which == 0) gat_hub_kernel<FT, VEC, GROUP, NACC, 0><<<hub_grid, ht, 0, s>>>(p);
+    else if (which == 1) gat_hub_kernel<FT, VEC, GROUP, NACC, 1><<<hub_grid, ht, 0, s>>>(p);
+    else gat_hub_kernel<FT, VEC, GROUP, NACC, 2><<<hub_grid, ht, 0, s>>>(p);
     STG_LAUNCH_CHECK("gat hub kernel");
   }
   if constexpr (GROUP == 32) {
@@ -693,44 +744,45 @@ int launch_gat(const GatParams& p, int which, cudaStream_t s) {
       if (p.queue != nullptr && gat_queue_chunk() > 0) {
         const int gblocks = std::min(sm_count() * (NACC == 1 ? 4 : 1), (p.num_rows + 7) / 8);
         const int ch = gat_queue_chunk();
-        if (which == 0) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 0, true>, gblocks, kGatThreads, s, hubs, p, ch));
-        else if (which == 1) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 1, true>, gblocks, kGatThreads, s, hubs, p, ch));
-        else STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 2, true>, gblocks, kGatThreads, s, hubs, p, ch));
+        if (which == 0) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 0, true>, gblocks, kGatThreads, s, hubs, p, ch));
+        else if (which == 1) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 1, true>, gblocks, kGatThreads, s, hubs, p, ch));
+        else STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 2, true>, gblocks, kGatThreads, s, hubs, p, ch));
         STG_LAUNCH_CHECK("gat rows (global queue) kernel");
         return STG_OK;
       }
       const int rpb = (kGatThreads / 32) * kGatRowsPerWarp;
       const int pblocks = (p.num_rows + rpb - 1) / rpb;
-      if (which == 0) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 0>, pblocks, kGatThreads, s, hubs, p, rpb));
-      else if (which == 1) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 1>, pblocks, kGatThreads, s, hubs, p, rpb));
-      else STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<VEC, NACC, 2>, pblocks, kGatThreads, s, hubs, p, rpb));
+      if (which == 0) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 0>, pblocks, kGatThreads, s, hubs, p, rpb));
+      else if (which == 1) STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 1>, pblocks, kGatThreads, s, hubs, p, rpb));
+      else STG_CUDA(launch_overlapped(gat_rows_pipe_kernel<FT, VEC, NACC, 2>, pblocks, kGatThreads, s, hubs, p, rpb));
       STG_LAUNCH_CHECK("gat rows (queue) kernel");
       return STG_OK;
     }
   }
-  if (which == 0) gat_fwd_kernel<VEC, GROUP, NACC><<<blocks, kGatThreads, 0, s>>>(p);
-  else if (which == 1) gat_bwd_kernel<VEC, GROUP, NACC, false><<<blocks, kGatThreads, 0, s>>>(p);
-  else gat_bwd_kernel<VEC, GROUP, NACC, true><<<blocks, kGatThreads, 0, s>>>(p);
+  if (which == 0) gat_fwd_kernel<FT, VEC, GROUP, NACC><<<blocks, kGatThreads, 0, s>>>(p);
+  else if (which == 1) gat_bwd_kernel<FT, VEC, GROUP, NACC, false><<<blocks, kGatThreads, 0, s>>>(p);
+  else gat_bwd_kernel<FT, VEC, GROUP, NACC, true><<<blocks, kGatThreads, 0, s>>>(p);
   STG_LAUNCH_CHECK("gat kernel");
   return STG_OK;
 }
 
-template <int VEC>
-int dispatch_gat(const GatParams& p, int which, cudaStream_t s) {
+template <typename FT, int VEC>
+int dispatch_gat(const GatParams<FT>& p, int which, cudaStream_t s) {
   const int nvec = p.hd / VEC;
-  if (nvec <= 1) return launch_gat<VEC, 1, 1>(p, which, s);
-  if (nvec <= 2) return launch_gat<VEC, 2, 1>(p, which, s);
-  if (nvec <= 4) return launch_gat<VEC, 4, 1>(p, which, s);
-  if (nvec <= 8) return launch_gat<VEC, 8, 1>(p, which, s);
-  if (nvec <= 16) return launch_gat<VEC, 16, 1>(p, which, s);
-  if (nvec <= 32) return launch_gat<VEC, 32, 1>(p, which, s);
-  if (nvec <= 64) return launch_gat<VEC, 32, 2>(p, which, s);
-  if (nvec <= 128) return launch_gat<VEC, 32, 4>(p, which, s);
+  if (nvec <= 1) return launch_gat<FT, VEC, 1, 1>(p, which, s);
+  if (nvec <= 2) return launch_gat<FT, VEC, 2, 1>(p, which, s);
+  if (nvec <= 4) return launch_gat<FT, VEC, 4, 1>(p, which, s);
+  if (nvec <= 8) return launch_gat<FT, VEC, 8, 1>(p, which, s);
+  if (nvec <= 16) return launch_gat<FT, VEC, 16, 1>(p, which, s);
+  if (nvec <= 32) return launch_gat<FT, VEC, 32, 1>(p, which, s);
+  if (nvec <= 64) return launch_gat<FT, VEC, 32, 2>(p, which, s);
+  if (nvec <= 128) return launch_gat<FT, VEC, 32, 4>(p, which, s);
   set_error("heads*dim = %d is wider than the fused GAT kernels support (512 floats with dim %% 4 == 0)", p.hd);
   return STG_ERR_UNSUPPORTED;
 }
 
-int run_gat(GatParams p, int which, bool aligned, cudaStream_t s) {
+template <typename FT>
+int run_gat(GatParams<FT> p, int which, bool aligned, cudaStream_t s) {
   const int vec = (p.dim % 4 == 0 && aligned) ? 4 : 1;
   p.lph = p.dim / vec;
   if ((p.lph & (p.lph - 1)) != 0 || p.lph > 32) {
@@ -738,7 +790,7 @@ int run_gat(GatParams p, int which, bool aligned, cudaStream_t s) {
               p.dim);
     return STG_ERR_UNSUPPORTED;
   }
-  return vec == 4 ? dispatch_gat<4>(p, which, s) : dispatch_gat<1>(p, which, s);
+  return vec == 4 ? dispatch_gat<FT, 4>(p, which, s) : dispatch_gat<FT, 1>(p, which, s);
 }
 
 int check_view(const StgCsrView* g) {
@@ -747,7 +799,8 @@ int check_view(const StgCsrView* g) {
   return STG_OK;
 }
 
-void bind_view(GatParams& p, const StgCsrView* g) {
+template <typename FT>
+void bind_view(GatParams<FT>& p, const StgCsrView* g) {
   p.row_off = g->row_offset;
   p.col = g->column_indices;
   p.queue = g->work_queue;
@@ -758,20 +811,21 @@ void bind_view(GatParams& p, const StgCsrView* g) {
   p.hub_capacity = hubs ? g->hub_capacity : 0;
 }
 
-}  // namespace
-}  // namespace stg
+// VEC = 4 needs four consecutive feat / d_feat elements to be one aligned access (16 bytes of fp32, 8 of 16-bit rows)
+template <typename FT>
+bool vec4_aligned(const void* p) {
+  return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(FT) - 1)) == 0;
+}
 
-using namespace stg;
-
-STG_API int stg_gat_softmax_fwd_f32(const StgCsrView* g_in, const float* el, const float* er, const float* feat,
-                                    int32_t heads, int32_t dim, float slope, float* out, float* row_max,
-                                    float* row_sum, void* stream) {
+template <typename FT>
+int gat_fwd(const StgCsrView* g_in, const float* el, const float* er, const FT* feat, int32_t heads, int32_t dim,
+            float slope, float* out, float* row_max, float* row_sum, void* stream) {
   int rc = check_view(g_in);
   if (rc != STG_OK) return rc;
   STG_CHECK_ARG(heads > 0 && dim > 0, "heads and dim must be positive");
   if (g_in->num_nodes == 0) return STG_OK;
   STG_CHECK_ARG(el && er && feat && out && row_max && row_sum, "NULL tensor");
-  GatParams p{};
+  GatParams<FT> p{};
   bind_view(p, g_in);
   p.num_rows = g_in->num_nodes;
   p.heads = heads;
@@ -784,13 +838,13 @@ STG_API int stg_gat_softmax_fwd_f32(const StgCsrView* g_in, const float* el, con
   p.row_max = row_max;
   p.row_sum = row_sum;
   p.o_vec = out;
-  return run_gat(p, 0, aligned16(feat) && aligned16(out), as_stream(stream));
+  return run_gat(p, 0, vec4_aligned<FT>(feat) && aligned16(out), as_stream(stream));
 }
 
-STG_API int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_out, const float* el, const float* er,
-                                    const float* feat, const float* out, const float* grad_out, const float* row_max,
-                                    const float* row_sum, int32_t heads, int32_t dim, float slope, float* d_feat,
-                                    float* d_el, float* d_er, float* dot_scratch, void* stream) {
+template <typename FT>
+int gat_bwd(const StgCsrView* g_in, const StgCsrView* g_out, const float* el, const float* er, const FT* feat,
+            const float* out, const float* grad_out, const float* row_max, const float* row_sum, int32_t heads,
+            int32_t dim, float slope, FT* d_feat, float* d_el, float* d_er, float* dot_scratch, void* stream) {
   int rc = check_view(g_in);
   if (rc != STG_OK) return rc;
   rc = check_view(g_out);
@@ -800,7 +854,7 @@ STG_API int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_
   if (g_in->num_nodes == 0) return STG_OK;
   STG_CHECK_ARG(el && er && feat && out && grad_out && row_max && row_sum && d_feat && d_el && d_er && dot_scratch,
                 "NULL tensor");
-  GatParams p{};
+  GatParams<FT> p{};
   p.num_rows = g_in->num_nodes;
   p.heads = heads;
   p.dim = dim;
@@ -814,7 +868,7 @@ STG_API int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_
   p.row_max = const_cast<float*>(row_max);
   p.row_sum = const_cast<float*>(row_sum);
   p.dot = dot_scratch;
-  const bool al = aligned16(feat) && aligned16(out) && aligned16(grad_out) && aligned16(d_feat);
+  const bool al = vec4_aligned<FT>(feat) && aligned16(out) && aligned16(grad_out) && vec4_aligned<FT>(d_feat);
   cudaStream_t s = as_stream(stream);
   // pass A: destination-parallel on the in-edge view -> dot, d_er
   bind_view(p, g_in);
@@ -824,7 +878,55 @@ STG_API int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_
   if (rc != STG_OK) return rc;
   // pass B: source-parallel on the out-edge view -> d_feat, d_el
   bind_view(p, g_out);
-  p.o_vec = d_feat;
+  p.o_vec = reinterpret_cast<float*>(d_feat);
   p.o_head = d_el;
   return run_gat(p, 2, al, s);
+}
+
+int check_dtype(int32_t dtype) {
+  STG_CHECK_ARG(dtype == STG_DTYPE_BF16 || dtype == STG_DTYPE_F16, "unknown dtype code %d (STG_DTYPE_BF16 = 1, STG_DTYPE_F16 = 2)",
+                dtype);
+  return STG_OK;
+}
+
+}  // namespace
+}  // namespace stg
+
+using namespace stg;
+
+STG_API int stg_gat_softmax_fwd_f32(const StgCsrView* g_in, const float* el, const float* er, const float* feat,
+                                    int32_t heads, int32_t dim, float slope, float* out, float* row_max,
+                                    float* row_sum, void* stream) {
+  return gat_fwd(g_in, el, er, feat, heads, dim, slope, out, row_max, row_sum, stream);
+}
+
+STG_API int stg_gat_softmax_bwd_f32(const StgCsrView* g_in, const StgCsrView* g_out, const float* el, const float* er,
+                                    const float* feat, const float* out, const float* grad_out, const float* row_max,
+                                    const float* row_sum, int32_t heads, int32_t dim, float slope, float* d_feat,
+                                    float* d_el, float* d_er, float* dot_scratch, void* stream) {
+  return gat_bwd(g_in, g_out, el, er, feat, out, grad_out, row_max, row_sum, heads, dim, slope, d_feat, d_el, d_er,
+                 dot_scratch, stream);
+}
+
+STG_API int stg_gat_softmax_fwd_h16(const StgCsrView* g_in, const float* el, const float* er, const void* feat,
+                                    int32_t heads, int32_t dim, int32_t dtype, float slope, float* out, float* row_max,
+                                    float* row_sum, void* stream) {
+  const int rc = check_dtype(dtype);
+  if (rc != STG_OK) return rc;
+  if (dtype == STG_DTYPE_BF16)
+    return gat_fwd(g_in, el, er, static_cast<const __nv_bfloat16*>(feat), heads, dim, slope, out, row_max, row_sum, stream);
+  return gat_fwd(g_in, el, er, static_cast<const __half*>(feat), heads, dim, slope, out, row_max, row_sum, stream);
+}
+
+STG_API int stg_gat_softmax_bwd_h16(const StgCsrView* g_in, const StgCsrView* g_out, const float* el, const float* er,
+                                    const void* feat, const float* out, const float* grad_out, const float* row_max,
+                                    const float* row_sum, int32_t heads, int32_t dim, int32_t dtype, float slope,
+                                    void* d_feat, float* d_el, float* d_er, float* dot_scratch, void* stream) {
+  const int rc = check_dtype(dtype);
+  if (rc != STG_OK) return rc;
+  if (dtype == STG_DTYPE_BF16)
+    return gat_bwd(g_in, g_out, el, er, static_cast<const __nv_bfloat16*>(feat), out, grad_out, row_max, row_sum, heads,
+                   dim, slope, static_cast<__nv_bfloat16*>(d_feat), d_el, d_er, dot_scratch, stream);
+  return gat_bwd(g_in, g_out, el, er, static_cast<const __half*>(feat), out, grad_out, row_max, row_sum, heads, dim,
+                 slope, static_cast<__half*>(d_feat), d_el, d_er, dot_scratch, stream);
 }
