@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define STG_ABI_VERSION 5
+#define STG_ABI_VERSION 6
 
 typedef enum StgStatus {
   STG_OK = 0,
@@ -355,6 +355,23 @@ int stg_tgcn_reset_bwd_f32(const float* p, const float* h, const float* d_hr, fl
 int stg_tgcn_update_fwd_f32(const float* p, const float* h, float* out, int64_t rows, int32_t hid, void* stream);
 int stg_tgcn_update_bwd_f32(const float* p, const float* h, const float* d_out, float* d_p, float* d_h, int64_t rows,
                             int32_t hid, void* stream);
+/* The 16-bit cell (torch.autocast): the tensors that only feed GEMMs are stored as bf16 / fp16 (dtype, StgDtype), the
+ * rest stays fp32; the arithmetic is the fp32 entry points', in fp32, and a value is rounded once, when it is stored.
+ *   bias_clamp_h16 : y = clamp(a + bias[c], lo, hi) with a and y [rows, cols] 16-bit, bias fp32 (may be NULL); y may be a;
+ *   clamp_bwd_h16  : d_a = d_y where lo < a + bias[c] < hi in fp32, else 0 (a, d_y, d_a 16-bit; d_a may be d_y) -- the
+ *                    fp32 cell's mask on the unrounded clamp input, which the rounded y cannot give (bf16: 1e6 -> 999424);
+ *   reset_fwd_h16  : stg_tgcn_reset_fwd_f32 with a 16-bit hr;
+ *   reset_bwd_h16, update_bwd_h16 : the fp32 entry points, and the blocks of d_p they write once more, rounded, into the
+ *                    16-bit [rows, 3*hid] d_p16. */
+int stg_tgcn_bias_clamp_h16(const void* a, const float* bias, void* y, int64_t rows, int32_t cols, int32_t dtype, float lo,
+                            float hi, void* stream);
+int stg_tgcn_clamp_bwd_h16(const void* a, const float* bias, const void* d_y, void* d_a, int64_t rows, int32_t cols,
+                           int32_t dtype, float lo, float hi, void* stream);
+int stg_tgcn_reset_fwd_h16(const float* p, const float* h, void* hr, int64_t rows, int32_t hid, int32_t dtype, void* stream);
+int stg_tgcn_reset_bwd_h16(const float* p, const float* h, const float* d_hr, float* d_p, void* d_p16, float* d_h,
+                           int64_t rows, int32_t hid, int32_t dtype, void* stream);
+int stg_tgcn_update_bwd_h16(const float* p, const float* h, const float* d_out, float* d_p, void* d_p16, float* d_h,
+                            int64_t rows, int32_t hid, int32_t dtype, void* stream);
 
 /* Weight-gradient GEMM of the cell: C[K, Nc] = A[M, K]^T * B[M, Nc] in exact fp32 for M >> K, Nc (what torch autograd
  * computes with cuBLAS for the gradients of conv_*.weight and linear_*.weight, tgcn.py:16-47), and, if colsum_b is not

@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STG_B200_LIB") or os.path.join(_HERE, "lib", "libstgraph_b200.so")   # env: A/B builds only
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 VM_MAX_TENSORS = 24
 VM_MAX_INSTR = 96
 VM_MAX_REGS = 48
@@ -141,6 +141,15 @@ _SIGNATURES = {
     "stg_tgcn_reset_bwd_f32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p], True),
     "stg_tgcn_update_fwd_f32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p], True),
     "stg_tgcn_update_bwd_f32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p], True),
+    "stg_tgcn_bias_clamp_h16": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_float, c_float,
+                                               c_void_p], True),
+    "stg_tgcn_clamp_bwd_h16": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_float,
+                                              c_float, c_void_p], True),
+    "stg_tgcn_reset_fwd_h16": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_void_p], True),
+    "stg_tgcn_reset_bwd_h16": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
+                                              c_int32, c_void_p], True),
+    "stg_tgcn_update_bwd_h16": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
+                                               c_int32, c_void_p], True),
     "stg_gemm_tn_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32], False),
     "stg_gemm_tn_f32": (ctypes.c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int32, c_int32, c_void_p, c_void_p,
                                        c_void_p, c_size_t, c_void_p], True),

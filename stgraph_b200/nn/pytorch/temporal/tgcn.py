@@ -105,15 +105,31 @@ class TGCN(torch.nn.Module):
         for t in packed:          # any gradient that reaches the pack means a backward pass has run through it
             if t.requires_grad:
                 t.register_hook(lambda grad, flag=stale: flag.__setitem__(0, True))
-        self.__dict__["_pack_cache"] = (key, packed, stale)
+        self.__dict__["_pack_cache"] = (key, packed, stale, {})
         return packed
+
+    def _lowp_parameters(self, packed, dt):
+        """The 16-bit GEMM operands of the pack (``ops_tgcn.lowp_parameters``), made once per pack and dtype and kept
+        beside it in ``_pack_cache``."""
+        from ....ops_tgcn import lowp_parameters
+
+        cache = self.__dict__.get("_pack_cache")
+        if cache is None or cache[1] is not packed:
+            return lowp_parameters(packed, dt)
+        if dt not in cache[3]:
+            cache[3][dt] = lowp_parameters(packed, dt)
+        return cache[3][dt]
 
     def _forward_fused(self, g, X, edge_weight, H):
         """The cell as ONE autograd op with a hand-written backward (``ops_tgcn``)."""
         from ....ops_tgcn import tgcn_cell
 
         norm = self._check_fused_inputs(g, edge_weight)
-        return tgcn_cell(g, X, H, norm, edge_weight, self._packed_parameters())
+        packed = self._packed_parameters()
+        lowp = None
+        if torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") in (torch.bfloat16, torch.float16):
+            lowp = self._lowp_parameters(packed, torch.get_autocast_dtype("cuda"))
+        return tgcn_cell(g, X, H, norm, edge_weight, packed, lowp)
 
     def _forward_fused_pieces(self, g, X, edge_weight, H):
         """The fused cell of round 1 (``fused="pieces"``): the same kernels, chained by torch autograd piece by piece."""
@@ -141,13 +157,16 @@ class TGCN(torch.nn.Module):
         norm = g.get_ndata("norm") if hasattr(g, "get_ndata") else None
         return (all(type(c) is GCNConv and c.activation is None and c.bias is not None for c in convs)
                 and not hasattr(g, "num_local_nodes") and norm is not None and not norm.requires_grad
-                and not torch.is_autocast_enabled("cuda")          # the one-op cell computes in float32 only
+                and (not torch.is_autocast_enabled("cuda")         # the one-op cell has an fp32 and a bf16 / fp16 form
+                     or torch.get_autocast_dtype("cuda") in (torch.bfloat16, torch.float16))
                 and (edge_weight is None or not edge_weight.requires_grad))
 
     def forward(self, g, X, edge_weight=None, H=None):
         if self.fused or (self.fused is None and self._can_fuse(g, edge_weight)):
             if H is None:      # allocated on the device directly: no H2D copy, CUDA-graph capturable
-                H = torch.zeros(X.shape[0], self.out_channels, device=X.device, dtype=X.dtype)
+                # under autocast the hidden state is fp32 (X is 16-bit when a model's own Linear feeds the cell)
+                dtype = torch.float32 if torch.is_autocast_enabled("cuda") else X.dtype
+                H = torch.zeros(X.shape[0], self.out_channels, device=X.device, dtype=dtype)
             if self.fused == "pieces":
                 return self._forward_fused_pieces(g, X, edge_weight, H)
             return self._forward_fused(g, X, edge_weight, H)

@@ -53,9 +53,22 @@ def _aggregate(csr, view, x, nflat, wflat):
     return kernels.agg_scaled_sum(view, x, nflat, wflat, nflat)
 
 
+def lowp_parameters(packed, dt):
+    """The 16-bit GEMM operands of :func:`pack_parameters`' tuple: ``(W3, La, Lc_zr, Lc_h)`` rounded to ``dt``, detached
+    (the cell returns the gradients of the fp32 pack).  Made once per pack, not per step."""
+    W3, _, La, Lc_zr, Lc_h, _ = packed
+    return tuple(t.detach().to(dt).contiguous() for t in (W3, La, Lc_zr, Lc_h))
+
+
 class _TgcnCell(torch.autograd.Function):
+    """``lowp`` is None (fp32 cell) or ``(dt, W3, La, Lc_zr, Lc_h)`` in ``dt`` = bf16 / fp16 (the cell under autocast)."""
+
     @staticmethod
-    def forward(ctx, fwd_view, bwd_view, keepalive, norm, edge_weight, X, H, W3, b3, La, Lc_zr, Lc_h, lb):
+    def forward(ctx, fwd_view, bwd_view, keepalive, norm, edge_weight, X, H, W3, b3, La, Lc_zr, Lc_h, lb, lowp):
+        ctx.lowp = lowp is not None
+        if lowp is not None:
+            with torch.autocast("cuda", enabled=False):
+                return _TgcnCell._forward16(ctx, fwd_view, bwd_view, keepalive, norm, edge_weight, X, H, b3, lb, lowp)
         X, H = X.contiguous(), H.contiguous()
         n, hid = H.shape
         st = _lib.current_stream_ptr()
@@ -81,6 +94,9 @@ class _TgcnCell(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, d_out):
+        if ctx.lowp:
+            with torch.autocast("cuda", enabled=False):
+                return _TgcnCell._backward16(ctx, d_out)
         X, H, h, P, HR, W3, La, Lc_zr, Lc_h, nflat, wflat = ctx.saved_tensors
         bwd_view, keepalive = ctx.views
         need = ctx.needs_input_grad          # (.., X=5, H=6, W3=7, b3=8, La=9, Lc_zr=10, Lc_h=11, lb=12)
@@ -131,17 +147,119 @@ class _TgcnCell(torch.autograd.Function):
                     kernels.gemm_tn(h[:, blk], dP[:, blk], out=d_La[g])
                 else:
                     torch.mm(h[:, blk].t(), dP[:, blk], out=d_La[g])
-        return (None, None, None, None, None, d_X, dH if need[6] else None, d_W3, d_b3, d_La, d_Lc_zr, d_Lc_h, d_lb)
+        return (None, None, None, None, None, d_X, dH if need[6] else None, d_W3, d_b3, d_La, d_Lc_zr, d_Lc_h, d_lb, None)
+
+    # ---- the cell under autocast (dt = bf16 / fp16).  Every GEMM takes dt operands and accumulates in fp32.  Stored in
+    # dt: X·W3, its aggregation A, h = clamp(A + b3), HR, the dt twin dP16 of dP, dh and dXW -- the tensors that are only
+    # GEMM operands -- each written by the kernel or GEMM that produces it.  Stored in fp32: P, out, dP, dH and the
+    # parameter gradients.  The gate arithmetic is the fp32 kernels' (csrc/gates.cu).
+    @staticmethod
+    def _forward16(ctx, fwd_view, bwd_view, keepalive, norm, edge_weight, X, H, b3, lb, lowp):
+        dt, W3, La, Lc_zr, Lc_h = lowp
+        f32 = torch.float32
+        code = kernels.H16_DTYPES[dt]
+        X16 = X.to(dt).contiguous()                        # X and H: one cast each (none when they come in dt / fp32)
+        H32 = H.to(f32).contiguous()
+        H16 = H.to(dt).contiguous()
+        n, hid = H.shape
+        st = _lib.current_stream_ptr()
+        nflat = norm.reshape(-1)
+        wflat = edge_weight.reshape(-1) if edge_weight is not None else None
+        b3 = b3.contiguous()
+        A = _aggregate(keepalive[0], fwd_view, torch.mm(X16, W3), nflat, wflat)        # [N, 3H] dt, kept for the mask
+        h = torch.empty_like(A)
+        _lib.call("stg_tgcn_bias_clamp_h16", A.data_ptr(), b3.data_ptr(), h.data_ptr(), n, 3 * hid, code, -CLAMP, CLAMP, st)
+        P = torch.empty(n, 3 * hid, device=H.device, dtype=f32)
+        torch.addmm(lb[:2 * hid], H16, Lc_zr, out_dtype=f32, out=P[:, :2 * hid])
+        for g in range(2):
+            blk = P[:, g * hid:(g + 1) * hid]
+            torch.addmm(blk, h[:, g * hid:(g + 1) * hid], La[g], out_dtype=f32, out=blk)
+        HR = torch.empty(n, hid, device=H.device, dtype=dt)
+        _lib.call("stg_tgcn_reset_fwd_h16", P.data_ptr(), H32.data_ptr(), HR.data_ptr(), n, hid, code, st)
+        Ph = P[:, 2 * hid:]
+        torch.addmm(lb[2 * hid:], HR, Lc_h, out_dtype=f32, out=Ph)
+        torch.addmm(Ph, h[:, 2 * hid:], La[2], out_dtype=f32, out=Ph)
+        out = torch.empty(n, hid, device=H.device, dtype=f32)
+        _lib.call("stg_tgcn_update_fwd_f32", P.data_ptr(), H32.data_ptr(), out.data_ptr(), n, hid, st)
+        kernels.launch_count += 3
+        ctx.views = (bwd_view, keepalive)
+        ctx.weighted = wflat is not None
+        ctx.dt, ctx.x_dtype = dt, X.dtype
+        ctx.save_for_backward(X16, H32, H16, A, h, P, HR, W3, b3, La, Lc_zr, Lc_h, nflat,
+                              wflat if wflat is not None else nflat)
+        return out
+
+    @staticmethod
+    def _backward16(ctx, d_out):
+        X16, H32, H16, A, h, P, HR, W3, b3, La, Lc_zr, Lc_h, nflat, wflat = ctx.saved_tensors
+        bwd_view, keepalive = ctx.views
+        need = ctx.needs_input_grad          # (.., X=5, H=6, W3=7, b3=8, La=9, Lc_zr=10, Lc_h=11, lb=12)
+        dt, f32 = ctx.dt, torch.float32
+        code = kernels.H16_DTYPES[dt]
+        n, hid = H32.shape
+        st = _lib.current_stream_ptr()
+        d_out = d_out.to(f32).contiguous()
+        dP = torch.empty_like(P)
+        dP16 = torch.empty(n, 3 * hid, device=P.device, dtype=dt)
+        dH = torch.empty_like(H32)
+        _lib.call("stg_tgcn_update_bwd_h16", P.data_ptr(), H32.data_ptr(), d_out.data_ptr(), dP.data_ptr(), dP16.data_ptr(),
+                  dH.data_ptr(), n, hid, code, st)
+        dHR = torch.mm(dP16[:, 2 * hid:], Lc_h.t(), out_dtype=f32)
+        _lib.call("stg_tgcn_reset_bwd_h16", P.data_ptr(), H32.data_ptr(), dHR.data_ptr(), dP.data_ptr(), dP16.data_ptr(),
+                  dH.data_ptr(), n, hid, code, st)
+        if need[6]:
+            torch.addmm(dH, dP16[:, :2 * hid], Lc_zr.t(), out_dtype=f32, out=dH)
+        dh = torch.empty_like(h)
+        for g in range(3):
+            torch.mm(dP16[:, g * hid:(g + 1) * hid], La[g].t(), out=dh[:, g * hid:(g + 1) * hid])
+        # gradient of clamp(A + b3): masked in place on the fp32 value A + b3, not on the rounded h
+        _lib.call("stg_tgcn_clamp_bwd_h16", A.data_ptr(), b3.data_ptr(), dh.data_ptr(), dh.data_ptr(), n, 3 * hid, code,
+                  -CLAMP, CLAMP, st)
+        kernels.launch_count += 3
+        d_b3 = dh.sum(0, dtype=f32) if need[8] else None
+
+        def tn(a, b, out=None):          # weight gradients [K, N] x [N, Nc]: dt operands, fp32 result, at every N
+            return torch.mm(a.t(), b, out_dtype=f32) if out is None else torch.mm(a.t(), b, out_dtype=f32, out=out)
+
+        d_W3 = d_X = None
+        if need[5] or need[7]:
+            dXW = _aggregate(keepalive[1], bwd_view, dh, nflat, wflat if ctx.weighted else None)
+            if need[7]:
+                d_W3 = tn(X16, dXW)
+            if need[5]:
+                d_X = torch.mm(dXW, W3.t()) if ctx.x_dtype == dt else torch.mm(dXW, W3.t(), out_dtype=f32)
+        d_lb = dP.sum(0) if need[12] else None
+        d_Lc_zr = tn(H16, dP16[:, :2 * hid]) if need[10] else None
+        d_Lc_h = tn(HR, dP16[:, 2 * hid:]) if need[11] else None
+        d_La = None
+        if need[9]:
+            d_La = torch.empty(La.shape, device=La.device, dtype=f32)
+            for g in range(3):
+                blk = slice(g * hid, (g + 1) * hid)
+                tn(h[:, blk], dP16[:, blk], out=d_La[g])
+        return (None, None, None, None, None, d_X, dH if need[6] else None, d_W3, d_b3, d_La, d_Lc_zr, d_Lc_h, d_lb, None)
 
 
-def tgcn_cell(graph, X, H, norm, edge_weight, packed):
+def tgcn_cell(graph, X, H, norm, edge_weight, packed, lowp=None):
     """One step of the TGCN cell on ``graph`` (static graph or the current snapshot of a dynamic one); ``packed`` is
-    :func:`pack_parameters`' tuple.  Differentiable w.r.t. ``X``, ``H`` and the packed parameters."""
+    :func:`pack_parameters`' tuple.  Differentiable w.r.t. ``X``, ``H`` and the packed parameters.
+
+    Under ``torch.autocast("cuda", dtype=dt)`` with ``dt`` bf16 / fp16 the cell runs its 16-bit form: ``X`` and ``H`` may
+    be fp32 or ``dt``, the GEMMs take ``dt`` operands (``lowp``: :func:`lowp_parameters` of ``packed``, made here when
+    None) with fp32 accumulation, and the returned hidden state is fp32."""
     if not X.is_cuda:
         raise RuntimeError("X must live on a CUDA device (stgraph_b200 has no CPU path)")
-    if X.dtype != torch.float32 or H.dtype != torch.float32:
+    lp = None
+    if torch.is_autocast_enabled("cuda"):
+        dt = torch.get_autocast_dtype("cuda")
+        if dt not in kernels.H16_DTYPES:
+            raise TypeError(f"the fused TGCN cell runs under autocast with bfloat16 or float16, not {dt}")
+        if X.dtype not in (torch.float32, dt) or H.dtype not in (torch.float32, dt):
+            raise TypeError(f"under {dt} autocast the fused TGCN cell takes float32 or {dt} X and H, got {X.dtype} and {H.dtype}")
+        lp = (dt,) + (tuple(lowp) if lowp is not None else lowp_parameters(packed, dt))
+    elif X.dtype != torch.float32 or H.dtype != torch.float32:
         raise TypeError("the fused TGCN cell computes in float32")
     bwd = graph.bwd_view()            # backward first: a dynamic graph builds both views in one go
     fwd = graph.fwd_view()
     keep = (graph._forward_graph, graph._backward_graph)
-    return _TgcnCell.apply(fwd, bwd, keep, norm, edge_weight, X, H, *packed)
+    return _TgcnCell.apply(fwd, bwd, keep, norm, edge_weight, X, H, *packed, lp)
