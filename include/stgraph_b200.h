@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define STG_ABI_VERSION 6
+#define STG_ABI_VERSION 7
 
 typedef enum StgStatus {
   STG_OK = 0,
@@ -117,7 +117,7 @@ int stg_agg_packed_sum_strided_f32(const StgCsrView* g, const StgEdgeMeta* meta,
  * The scales and the packed records stay fp32; every product and the running sum are fp32, and each output element is
  * rounded to the 16-bit type once.  Assign mode only.  A graph's packed array (stg_csr_pack_edge_meta_f32) serves the
  * fp32 and the 16-bit entry points alike, and the packed sums equal the plain ones bit for bit.  feat == 0 is a no-op. */
-typedef enum StgDtype { STG_DTYPE_BF16 = 1, STG_DTYPE_F16 = 2 } StgDtype;
+typedef enum StgDtype { STG_DTYPE_F32 = 0, STG_DTYPE_BF16 = 1, STG_DTYPE_F16 = 2 } StgDtype;
 int stg_agg_scaled_sum_h16(const StgCsrView* g, const void* x, int32_t feat, int32_t dtype,
                            const float* nbr_scale, const float* edge_scale, const float* row_scale,
                            void* out, void* stream);
@@ -290,7 +290,7 @@ typedef struct StgVmTensor {
   int32_t side; /* StgVmSide */
   int32_t bc0;
   int32_t bc1;
-  int32_t pad;
+  int32_t dtype; /* StgDtype of the bound tensor: STG_DTYPE_F32 (0) for stg_vm_run_f32 */
 } StgVmTensor;
 
 typedef struct StgVmInstr {
@@ -314,6 +314,14 @@ typedef struct StgVmProgram {
 /* Runs the program once per (row, lane) of the given view (rows = "center" side). Tensors written
  * with a reducing STORE must be zero-filled by the caller (atomic accumulation may be used). */
 int stg_vm_run_f32(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream);
+/* The same program with bf16 / fp16 tensors among its inputs (torch.autocast): tensors[i] is stored as
+ * prog->tensors[i].dtype says.  A LOAD widens each element to fp32; registers, accumulators, arithmetic and every STORE
+ * target stay fp32 (a STORE to a 16-bit tensor is rejected).  The lanes are those of stg_vm_run_f32 with the alignment
+ * taken in elements (4 elements per lane when dim1 % 4 == 0 and every tensor read along dim1 is aligned to 4 of its
+ * elements: 16 bytes for fp32, 8 for 16-bit), so the results equal those of stg_vm_run_f32 on the widened tensors bit
+ * for bit.  It makes stg_vm_run_f32's checks with the same messages and rejects unknown dtype codes before any launch;
+ * stg_vm_run_f32 rejects any code but STG_DTYPE_F32. */
+int stg_vm_run_mixed(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream);
 
 /* ------------------------------------------------ link-prediction decode */
 /* out[p] = sum_f z[a[p], f] * z[b[p], f] for p < n_pairs (a, b: int64 vertex ids, z: [N, feat] fp32).

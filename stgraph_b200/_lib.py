@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STG_B200_LIB") or os.path.join(_HERE, "lib", "libstgraph_b200.so")   # env: A/B builds only
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 VM_MAX_TENSORS = 24
 VM_MAX_INSTR = 96
 VM_MAX_REGS = 48
@@ -44,7 +44,7 @@ class StgCsrView(Structure):
 
 
 class StgVmTensor(Structure):
-    _fields_ = [("side", c_int32), ("bc0", c_int32), ("bc1", c_int32), ("pad", c_int32)]
+    _fields_ = [("side", c_int32), ("bc0", c_int32), ("bc1", c_int32), ("dtype", c_int32)]
 
 
 class StgVmInstr(Structure):
@@ -128,6 +128,7 @@ _SIGNATURES = {
                                                c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_float,
                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p], True),
     "stg_vm_run_f32": (ctypes.c_int, [_P(StgCsrView), _P(StgVmProgram), _P(c_void_p), c_void_p], True),
+    "stg_vm_run_mixed": (ctypes.c_int, [_P(StgCsrView), _P(StgVmProgram), _P(c_void_p), c_void_p], True),
     "stg_edge_dot_f32": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_void_p, c_void_p], True),
     "stg_edge_dot_bwd_f32": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p], True),
     "stg_bias_clamp_f32": (ctypes.c_int, [c_void_p, c_void_p, c_int64, c_int32, c_float, c_float, c_void_p], True),

@@ -29,6 +29,9 @@ from .lowering import lower_unit
 from .registry import torch_eval
 from .utils import ValType, is_const_scalar
 
+#: ``StgDtype`` codes of the tensors a VM launch reads (``stg_vm_run_mixed``); it writes fp32 only
+_VM_DTYPE_CODES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
+
 
 class Stack:
     def __init__(self):
@@ -184,9 +187,12 @@ class Executor:
     def _alloc_unit_outputs(self, unit, tensor_map):
         needs_zero = set()
         written = set()
+        vm_written = set()
         for la in unit.launches:
             needs_zero |= la.needs_zero
             written |= set(la.writes)
+            if la.kind == "vm":
+                vm_written |= set(la.writes)
             # A scaled sum over bf16 / fp16 rows writes rows of that type.  The traced program cannot say so: it types
             # ``h * norm`` by promotion (fp32) and a gradient by its first operand, so the output takes x's dtype here.
             if la.kind == "scaled_sum" and la.out.id not in tensor_map:
@@ -195,7 +201,10 @@ class Executor:
                     tensor_map[la.out.id] = self._alloc(la.out, False, tensor_map, dtype=x.dtype)
         for var in unit.unit_rets():
             if var.id not in tensor_map:
-                tensor_map[var.id] = self._alloc(var, var in needs_zero or var not in written, tensor_map)
+                # The VM kernel writes fp32 whatever it reads.  The tracer types a statement by its first operand, so with
+                # a 16-bit input some intermediates and gradients are typed 16-bit: such a buffer would be half the size.
+                dtype = torch.float32 if var in vm_written else None
+                tensor_map[var.id] = self._alloc(var, var in needs_zero or var not in written, tensor_map, dtype=dtype)
 
     def execute_compiled(self, uid, FuncWrapper):
         mu = self.forward_exec_units[uid]
@@ -228,15 +237,24 @@ class Executor:
                                        out=tensor_map[la.out.id])
             return
         ptrs = (ctypes.c_void_p * _lib.VM_MAX_TENSORS)()
+        # The storage type of each tensor is the one bound at this launch: node-wise torch units and autocast decide it at
+        # run time, so the lowered program cannot carry it.
+        mixed = False
         for i, v in enumerate(la.tensor_vars):
             t = tensor_map[v.id]
             if not t.is_contiguous():
                 t = t.contiguous()
                 tensor_map[v.id] = t
-            if t.dtype != torch.float32:
-                raise TypeError(f"vertex-program tensors must be float32 (got {t.dtype} for {v.id})")
+            code = _VM_DTYPE_CODES.get(t.dtype)
+            if code is None:
+                raise TypeError(f"vertex-program tensors must be float32, bfloat16 or float16 (got {t.dtype} for {v.id})")
+            if code and v in la.writes:
+                raise TypeError(f"vertex-program outputs are float32 (got {t.dtype} for {v.id})")
+            la.program.tensors[i].dtype = code
+            mixed = mixed or code != 0
             ptrs[i] = self.raw_ptr(t) if self.raw_ptr is not None else ctypes.c_void_p(t.data_ptr())
-        _lib.call("stg_vm_run_f32", ctypes.byref(view), ctypes.byref(la.program), ptrs, _lib.current_stream_ptr())
+        _lib.call("stg_vm_run_mixed" if mixed else "stg_vm_run_f32", ctypes.byref(view), ctypes.byref(la.program), ptrs,
+                  _lib.current_stream_ptr())
         kernels.launch_count += 1
 
     def forward_cb(self, uid, kernel_args, rets, tensor_list):

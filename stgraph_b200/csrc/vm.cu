@@ -15,7 +15,12 @@
 // Virtual registers live in shared memory ([reg][thread], conflict-free); a register holds four consecutive
 // elements (float4) when the unit's inner dimension allows it.
 // This is the generality path; hot shapes are matched to agg.cu / gat.cu first.
+//
+// The mixed form (MIXED = true, stg_vm_run_mixed) also reads bf16 / fp16 tensors: LOAD widens each element to fp32 as
+// it is loaded, and registers, accumulators, arithmetic and every stored tensor stay fp32.  Its lanes are those of the
+// fp32 form on the widened tensors, so it computes the fp32 program's operations in the same order.
 #include "common.cuh"
+#include "h16.cuh"
 
 #include <type_traits>
 
@@ -75,6 +80,26 @@ template <> struct Vec<4> {
   }
 };
 
+// A 16-bit LOAD of the mixed form: one 8-byte load of 4 elements for a float4 register read along dim1 (wide), else one
+// 2-byte load, splatted when the tensor is broadcast along dim1.
+template <int VEC>
+__device__ __forceinline__ typename Vec<VEC>::T load_h16(const unsigned short* p, bool wide, bool bf16) {
+  if constexpr (VEC == 4) {
+    if (wide) {
+      const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+      float f[4];
+      if (bf16) unpack<__nv_bfloat16, 4>(r, f);
+      else unpack<__half, 4>(r, f);
+      return make_float4(f[0], f[1], f[2], f[3]);
+    }
+  }
+  const unsigned short r = __ldg(p);
+  float f[1];
+  if (bf16) unpack<__nv_bfloat16, 1>(r, f);
+  else unpack<__half, 1>(r, f);
+  return Vec<VEC>::splat(f[0]);
+}
+
 // HUB = false: one lane group per row (rows longer than the VM's hub threshold are skipped).
 // HUB = true : one BLOCK per hub row; every (warp, group) slot takes a strided share of the row's edges,
 //              the accumulators are merged through shared memory by kind (sum / max / min) in a fixed
@@ -84,7 +109,9 @@ template <> struct Vec<4> {
 // cannot overlap the instruction after it) and the decode cost is paid once per U edges.  Slot u of a register is
 // private to edge u of the batch; PRE runs for every slot (row-level values), POST for slot 0 after the
 // accumulators of the U slots have been merged in a fixed order.
-template <int GROUP, bool HUB, int VEC, int U>
+// MIXED = true: a LOAD reads its tensor in the type its StgVmTensor::dtype names (the same code for every lane, so the
+// branch is uniform); MIXED = false is the fp32 kernel.
+template <int GROUP, bool HUB, int VEC, int U, bool MIXED>
 __global__ void __launch_bounds__(HUB ? HubThreads<VEC>::value : kVmThreads)
     vm_kernel(const __grid_constant__ VmArgs a, const __grid_constant__ StgVmProgram prog) {
   using V = Vec<VEC>;
@@ -159,6 +186,27 @@ __global__ void __launch_bounds__(HUB ? HubThreads<VEC>::value : kVmThreads)
       switch (in.op) {
         case STG_OP_LOAD: {
           const StgVmTensor& t = prog.tensors[in.a];
+          if constexpr (MIXED) {
+            if (t.dtype != STG_DTYPE_F32) {
+              const bool bf16 = t.dtype == STG_DTYPE_BF16;
+              const unsigned short* base = static_cast<const unsigned short*>(a.tensors[in.a]);
+              const int tsz = tensor_size(t, prog.dim0, dim1), tel = tensor_elem(t, i0, i1, dim1);
+              T v[NU];
+#pragma unroll
+              for (int u = 0; u < NU; ++u) {
+                long long id = 0;
+                if (t.side == STG_VM_CENTER) id = row;
+                else if (t.side == STG_VM_NBR) id = nbr[u];
+                else if (t.side == STG_VM_EDGE) id = eid[u];
+                const unsigned short* src = base + id * tsz + tel;     // in elements of 2 bytes
+                v[u] = V::splat(0.f);
+                if (valid[u]) v[u] = load_h16<VEC>(src, t.bc1, bf16);
+              }
+#pragma unroll
+              for (int u = 0; u < NU; ++u) R(in.dst) = v[u];
+              break;
+            }
+          }
           const float* base = static_cast<const float*>(a.tensors[in.a]);
           const int tsz = tensor_size(t, prog.dim0, dim1), tel = tensor_elem(t, i0, i1, dim1);
           T v[NU];
@@ -300,7 +348,7 @@ __global__ void __launch_bounds__(HUB ? HubThreads<VEC>::value : kVmThreads)
 #undef ACC
 }
 
-template <int GROUP, int VEC, int U>
+template <int GROUP, int VEC, int U, bool MIXED>
 int launch_vm_rows(const VmArgs& a, const StgVmProgram& prog, cudaStream_t stream) {
   const int rows_per_block = (kVmThreads / 32) * (32 / GROUP);
   const int blocks = (a.g.num_nodes + rows_per_block - 1) / rows_per_block;
@@ -308,27 +356,27 @@ int launch_vm_rows(const VmArgs& a, const StgVmProgram& prog, cudaStream_t strea
   const size_t smem = per_thread * kVmThreads;
   static size_t configured = 48 * 1024;
   if (smem > configured) {
-    STG_CUDA(cudaFuncSetAttribute(vm_kernel<GROUP, false, VEC, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    STG_CUDA(cudaFuncSetAttribute(vm_kernel<GROUP, false, VEC, U, MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(smem)));
     configured = smem;
   }
-  vm_kernel<GROUP, false, VEC, U><<<blocks, kVmThreads, smem, stream>>>(a, prog);
+  vm_kernel<GROUP, false, VEC, U, MIXED><<<blocks, kVmThreads, smem, stream>>>(a, prog);
   STG_LAUNCH_CHECK("vm_kernel");
   return STG_OK;
 }
 
-template <int GROUP, int VEC, int U>
+template <int GROUP, int VEC, int U, bool MIXED>
 int launch_vm_hub(const VmArgs& a, const StgVmProgram& prog, cudaStream_t stream) {
   constexpr int ht = HubThreads<VEC>::value;
   const size_t per_thread = static_cast<size_t>(prog.n_regs + prog.n_acc) * U * VEC * sizeof(float) + sizeof(float);
   const size_t hub_smem = per_thread * ht;
   static size_t configured = 48 * 1024;
   if (hub_smem > configured) {
-    STG_CUDA(cudaFuncSetAttribute(vm_kernel<GROUP, true, VEC, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    STG_CUDA(cudaFuncSetAttribute(vm_kernel<GROUP, true, VEC, U, MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(hub_smem)));
     configured = hub_smem;
   }
-  vm_kernel<GROUP, true, VEC, U><<<(VEC == 4 ? 4 : 2) * sm_count(), ht, hub_smem, stream>>>(a, prog);
+  vm_kernel<GROUP, true, VEC, U, MIXED><<<(VEC == 4 ? 4 : 2) * sm_count(), ht, hub_smem, stream>>>(a, prog);
   STG_LAUNCH_CHECK("vm_kernel(hub)");
   return STG_OK;
 }
@@ -337,40 +385,36 @@ int launch_vm_hub(const VmArgs& a, const StgVmProgram& prog, cudaStream_t stream
 // kernel gains from U = 4 only with scalar lanes (a float4 register file is already 16 bytes per access and most rows
 // are shorter than a batch), the block-per-row kernel only with float4 lanes (long rows, latency-bound).  The
 // float4 hub kernel falls back to 2 / 1 when its register file would not fit shared memory.
-template <int GROUP, int VEC>
+template <int GROUP, int VEC, bool MIXED>
 int launch_vm(const VmArgs& a, const StgVmProgram& prog, cudaStream_t stream) {
   int rc;
-  if constexpr (VEC == 4) rc = launch_vm_rows<GROUP, 4, 1>(a, prog, stream);
-  else rc = launch_vm_rows<GROUP, 1, 4>(a, prog, stream);
+  if constexpr (VEC == 4) rc = launch_vm_rows<GROUP, 4, 1, MIXED>(a, prog, stream);
+  else rc = launch_vm_rows<GROUP, 1, 4, MIXED>(a, prog, stream);
   if (rc != STG_OK) return rc;
   if (a.g.num_edges <= kVmHubThreshold) return STG_OK;     // a row longer than the threshold cannot exist
   if constexpr (VEC == 4) {
     const size_t slot_bytes = static_cast<size_t>(prog.n_regs + prog.n_acc) * 16 * HubThreads<4>::value;
-    if (4 * slot_bytes <= 160 * 1024) return launch_vm_hub<GROUP, 4, 4>(a, prog, stream);
-    if (2 * slot_bytes <= 160 * 1024) return launch_vm_hub<GROUP, 4, 2>(a, prog, stream);
-    return launch_vm_hub<GROUP, 4, 1>(a, prog, stream);
+    if (4 * slot_bytes <= 160 * 1024) return launch_vm_hub<GROUP, 4, 4, MIXED>(a, prog, stream);
+    if (2 * slot_bytes <= 160 * 1024) return launch_vm_hub<GROUP, 4, 2, MIXED>(a, prog, stream);
+    return launch_vm_hub<GROUP, 4, 1, MIXED>(a, prog, stream);
   } else {
-    return launch_vm_hub<GROUP, 1, 1>(a, prog, stream);
+    return launch_vm_hub<GROUP, 1, 1, MIXED>(a, prog, stream);
   }
 }
 
-template <int VEC>
+template <int VEC, bool MIXED>
 int dispatch_vm(const VmArgs& a, const StgVmProgram& prog, cudaStream_t s) {
   const int lanes = prog.dim0 * prog.dim1 / VEC;
-  if (lanes <= 1) return launch_vm<1, VEC>(a, prog, s);
-  if (lanes <= 2) return launch_vm<2, VEC>(a, prog, s);
-  if (lanes <= 4) return launch_vm<4, VEC>(a, prog, s);
-  if (lanes <= 8) return launch_vm<8, VEC>(a, prog, s);
-  if (lanes <= 16) return launch_vm<16, VEC>(a, prog, s);
-  return launch_vm<32, VEC>(a, prog, s);
+  if (lanes <= 1) return launch_vm<1, VEC, MIXED>(a, prog, s);
+  if (lanes <= 2) return launch_vm<2, VEC, MIXED>(a, prog, s);
+  if (lanes <= 4) return launch_vm<4, VEC, MIXED>(a, prog, s);
+  if (lanes <= 8) return launch_vm<8, VEC, MIXED>(a, prog, s);
+  if (lanes <= 16) return launch_vm<16, VEC, MIXED>(a, prog, s);
+  return launch_vm<32, VEC, MIXED>(a, prog, s);
 }
 
-}  // namespace
-}  // namespace stg
-
-using namespace stg;
-
-STG_API int stg_vm_run_f32(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream) {
+// The argument checks of both entry points, then the launch.  mixed = false: every tensor must be fp32.
+int vm_run(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream, bool mixed) {
   STG_CHECK_ARG(g && prog && tensors, "NULL argument");
   STG_CHECK_ARG(g->row_offset != nullptr, "row_offset is NULL");
   STG_CHECK_ARG(prog->dim0 > 0 && prog->dim1 > 0, "program dims must be positive");
@@ -394,6 +438,22 @@ STG_API int stg_vm_run_f32(const StgCsrView* g, const StgVmProgram* prog, void* 
       STG_CHECK_ARG(d1 <= 32, "GSUM needs dim1 <= 32 (got %d)", d1);
     }
   }
+  for (int i = 0; i < prog->n_tensors; ++i) {
+    const int code = prog->tensors[i].dtype;
+    if (mixed) {
+      STG_CHECK_ARG(code == STG_DTYPE_F32 || code == STG_DTYPE_BF16 || code == STG_DTYPE_F16,
+                    "unknown dtype code %d of tensor %d (STG_DTYPE_F32 = 0, STG_DTYPE_BF16 = 1, STG_DTYPE_F16 = 2)", code, i);
+    } else {
+      STG_CHECK_ARG(code == STG_DTYPE_F32, "tensor %d has dtype code %d: stg_vm_run_f32 takes fp32 tensors only "
+                    "(16-bit tensors go to stg_vm_run_mixed)", i, code);
+    }
+  }
+  for (int i = 0; i < prog->n_instr; ++i) {
+    const StgVmInstr& in = prog->instr[i];
+    STG_CHECK_ARG(in.op != STG_OP_STORE || prog->tensors[in.a].dtype == STG_DTYPE_F32,
+                  "STORE at instr %d writes tensor %d with dtype code %d: the VM writes fp32 tensors only", i, in.a,
+                  prog->tensors[in.a].dtype);
+  }
   STG_CHECK_ARG(!needs_eids || g->eids_identity || g->eids || g->num_edges == 0, "eids is NULL");
   if (g->num_nodes == 0) return STG_OK;
   STG_CHECK_ARG(g->num_edges == 0 || g->column_indices, "column_indices is NULL");
@@ -402,12 +462,28 @@ STG_API int stg_vm_run_f32(const StgCsrView* g, const StgVmProgram* prog, void* 
   for (int i = 0; i < STG_VM_MAX_TENSORS; ++i) a.tensors[i] = i < prog->n_tensors ? tensors[i] : nullptr;
   cudaStream_t s = as_stream(stream);
   // float4 lanes when the four elements of a lane share their dim0 index and every tensor that is indexed along
-  // dim1 is 16-byte aligned (its per-row size is then a multiple of 4 floats)
+  // dim1 is aligned to four of its elements (16 bytes for fp32, 8 for 16-bit; its per-row size is then a multiple of 4
+  // elements).  A 16-bit view and an fp32 view at the same element offset therefore choose the same lanes.
   bool vec4 = prog->dim1 % 4 == 0;
-  for (int i = 0; vec4 && i < prog->n_tensors; ++i)
-    if (prog->tensors[i].bc1 && tensors[i] != nullptr && !aligned16(tensors[i])) vec4 = false;
+  for (int i = 0; vec4 && i < prog->n_tensors; ++i) {
+    const bool f32 = prog->tensors[i].dtype == STG_DTYPE_F32;
+    if (prog->tensors[i].bc1 && tensors[i] != nullptr && !(f32 ? aligned16(tensors[i]) : aligned8(tensors[i]))) vec4 = false;
+  }
   // the largest float4 register file the hub block may need must fit one SM's shared memory
   const size_t hub_bytes = (static_cast<size_t>(prog->n_regs + prog->n_acc) * 16 + 4) * HubThreads<4>::value;
-  if (vec4 && hub_bytes <= 200 * 1024) return dispatch_vm<4>(a, *prog, s);
-  return dispatch_vm<1>(a, *prog, s);
+  if (vec4 && hub_bytes <= 200 * 1024) return mixed ? dispatch_vm<4, true>(a, *prog, s) : dispatch_vm<4, false>(a, *prog, s);
+  return mixed ? dispatch_vm<1, true>(a, *prog, s) : dispatch_vm<1, false>(a, *prog, s);
+}
+
+}  // namespace
+}  // namespace stg
+
+using namespace stg;
+
+STG_API int stg_vm_run_f32(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream) {
+  return vm_run(g, prog, tensors, stream, false);
+}
+
+STG_API int stg_vm_run_mixed(const StgCsrView* g, const StgVmProgram* prog, void* const* tensors, void* stream) {
+  return vm_run(g, prog, tensors, stream, true);
 }

@@ -13,8 +13,9 @@ That behaviour is reproduced, not fixed.
 recompute-alpha backward, no ``[E,H]`` tensor and no atomics) on the hand-written kernels of
 ``csrc/gat.cu`` -- validated against a closed-form torch oracle, not against the reference.
 
-Under ``torch.autocast`` the projection ``fc(feat)`` is bf16 / fp16.  The fused op reads it as it is (fp32 softmax and
-output); the stock program runs on its fp32 widening.  Either way the output is fp32.
+Under ``torch.autocast`` the projection ``fc(feat)`` is bf16 / fp16.  The fused op and the stock program both read it as
+it is and widen each element on load (fp32 softmax and output); the output is fp32 and the projection's gradient is
+rounded to its dtype once.
 """
 from __future__ import annotations
 
@@ -86,9 +87,7 @@ class GATConv(nn.Module):
 
             out = gat_edge_softmax_aggregate(graph, left, right, proj, self.negative_slope)
         else:
-            # Under autocast proj is bf16 / fp16; the stock program is the fp32 VM path, so it gets the widened rows (the
-            # trace signature, and so the compiled program, is the fp32 one) and autograd casts the gradient back.
-            if proj.dtype in (torch.bfloat16, torch.float16):
-                proj = proj.float()
+            # Under autocast proj is bf16 / fp16 (el / er are fp32 by promotion): the VM reads it as it is, computes what
+            # it computes on proj.float(), and the fp32 gradient it returns is rounded to proj's dtype by autograd.
             out = self._stock_program()(g=graph, n_feats={"el": left, "er": right, "feat_src": proj})
         return self.activation(out) if self.activation else out
